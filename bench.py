@@ -2,7 +2,7 @@
 """Benchmark of the Graphical-Normalizing-Flows hot path on B200 (contract: see the task statement).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--config cfg1..cfg5] [--batch B_per_gpu] [--mode train|eval]
+                    [--config cfg1..cfg5] [--batch B_per_gpu] [--mode train|eval] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic input:
   train: zero_grad -> forward -> loss -> backward -> (gradient all-reduce if N>1) -> Adam step
@@ -202,6 +202,26 @@ def cpu_reference_step_fn(cfg, B, mode, S):
     return (train_step if mode == "train" else eval_step), "port"
 
 
+DUMP_BYTES = 64_000_000 - 64 * 1024             # all .npy files of --dump-outputs together, headers included
+
+
+def dump_outputs(outputs, out_dir):
+    """Write {name: tensor} as out_dir/<name>.npy in float32.  When the arrays together exceed DUMP_BYTES, every array keeps the
+    same fraction of its elements: a flat sample at sorted indices drawn from a fixed seed, so that two runs with the same
+    arguments store the same elements."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(t.numel() for t in outputs.values()) * 4
+    frac = min(1., DUMP_BYTES / max(total, 1))
+    for name, t in outputs.items():
+        t = t.detach().float().cpu()
+        if frac < 1.:
+            n = t.numel()
+            idx = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:max(1, int(n * frac))].sort().values
+            t = t.flatten()[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), t.numpy())
+
+
 def time_cpu(cfg, B, mode, S, steps, warmup, budget_s=25.):
     """Bounded CPU timing: EXACTLY `steps` timed steps after `warmup` untimed ones; the batch is reduced (stated in `sample`)
     when full-batch steps would blow the time budget."""
@@ -261,7 +281,13 @@ def main():
     ap.add_argument("--no-eval", action="store_true", help="train mode: skip the additional log-lik eval measurement")
     ap.add_argument("--cuda-graph", default="auto", choices=["auto", "on", "off"],
                     help="replay the training step (incl. the NCCL gradient all-reduce) as one captured CUDA graph (auto = on)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last device-timed step returned as DIR/<name>.npy (float32, at "
+                         "most 64 MB in all): train = loss and the parameter gradients; eval (and the eval measurement of a train "
+                         "run, prefixed eval.) = ll and z")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
 
@@ -283,6 +309,7 @@ def main():
     config["umnn_engine"] = args.umnn_engine
     config["cuda_graph"] = args.cuda_graph in ("on", "auto")
     config["allreduce"] = args.allreduce
+    config["timed_train_step"] = "from the seeded initial parameters and optimizer state"
     if args.random_steps:
         config["nb_steps"] = f"{S}+U{{0..9}} per step (UCIExperiments.py:131-133)"
 
@@ -316,6 +343,23 @@ def main():
         config["allreduce"] = "peer" if bucket.peer is not None else ("single" if world > 1 else "peer")
     # the reference's optimizer (torch.optim.Adam(lr, weight_decay), UCIExperiments.py:100) as one multi-tensor launch per step
     opt = G.FusedAdam(model.parameters(), lr=lr, weight_decay=wd)
+    # Every device-timed training step starts from the seeded initial parameters and a fresh optimizer state.  Several kernels
+    # sum with float atomics; from one state a step reproduces to rounding, but over a chain of Adam steps those last-bit
+    # differences grow until two runs with the same arguments no longer train the same model.  The restore runs between the
+    # timed steps, outside their events.
+    params = list(model.parameters())
+    init_params = [p.detach().clone() for p in params]
+
+    def restore_initial_state():
+        with torch.no_grad():
+            torch._foreach_copy_(params, init_params)
+            moments = [t for st in opt.state.values() for t in (st["exp_avg"], st["exp_avg_sq"])]
+            if moments:
+                torch._foreach_zero_(moments)
+            for group in opt.param_groups:
+                if "step" in group:
+                    group["step"].zero_()
+
     gen = torch.Generator(device=dev).manual_seed(1000 + rank)
     n_pool = 8
     pool = [torch.randn(B, d, device=dev, generator=gen) for _ in range(n_pool)]
@@ -346,9 +390,12 @@ def main():
         opt.step()
         return loss
 
+    last_eval = {}                    # (ll, z) of the latest eager evaluation step, for --dump-outputs
+
     def eval_step(x):
         with torch.no_grad():
-            ll, _ = model.compute_ll(x)
+            ll, z = model.compute_ll(x)
+        last_eval["ll"], last_eval["z"] = ll, z
         return ll.mean()
 
     def barrier():
@@ -357,12 +404,14 @@ def main():
         torch.cuda.synchronize()
 
     def measure(mode, precision, gemm, S_, steps, warmup, sample_clocks, use_graph=False):
-        """One arm: W warm-up steps, K device-timed steps (CUDA events per step, L2 flushed between steps), then K
-        end-to-end steps (pinned host batch -> H2D -> step -> loss D2H).  Max over ranks.
+        """One arm: W warm-up steps, K device-timed steps (CUDA events per step, L2 flushed between steps; a training step
+        starts from the seeded initial state), then K end-to-end steps (pinned host batch -> H2D -> step -> loss D2H).  Max
+        over ranks.
         use_graph: the timed steps replay ONE captured CUDA graph of the whole training step; the per-kernel times for
         the roofline object are then taken from a short eager pass first (a replay has no per-launch host hooks)."""
         G.ops.set_gemm_mode(gemm)
         G.ops.UMNN_ENGINE = args.umnn_engine
+        restore_initial_state()                # the eval arm of a train run evaluates the seeded model, not the trained one
         for n in model.getNormalizers():
             if hasattr(n, "nb_steps"):
                 n.nb_steps = S_
@@ -423,14 +472,27 @@ def main():
             G.ops.enable_kernel_timing(True)
         evs = []
         barrier()
+        out = None
         for i in range(steps):
+            if mode == "train":
+                restore_initial_state()
             flush_buf.zero_()
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
-            step(pool[i % n_pool])
+            out = step(pool[i % n_pool])
             e1.record()
             evs.append((e0, e1))
         barrier()
+        outputs = None
+        if args.dump_outputs:
+            # what the last device-timed step handed its caller, copied before the end-to-end steps overwrite it
+            if mode == "train":
+                outputs = {"loss": out}
+                outputs.update({"grad." + name: p.grad for name, p in model.named_parameters() if p.grad is not None})
+            else:
+                ll, z = graphed_eval.static_out if use_graph else (last_eval["ll"], last_eval["z"])
+                outputs = {"ll": ll, "z": z}
+            outputs = {k: v.detach().float().cpu() for k, v in outputs.items()}
         if use_graph:
             launches, ktimes, kflops, kshapes = eager_launches * steps, eager_ktimes, eager_kflops, eager_kshapes
         else:
@@ -565,7 +627,7 @@ def main():
                 "gpu_launches": launches, "clocks": clocks, "roofline": roofline,
                 "achieved_tflops_step": flops_step / (dev_ms / steps / 1e3) / 1e12, "algorithmic_gflop_per_step": flops_step / 1e9,
                 "last_loss": last, "kernel_ms": {k: sum(v) / len(v) for k, v in ktimes.items() if v},
-                "nb_steps": S_, "precision": precision, "gemm_engine": gemm, "cuda_graph": bool(use_graph)}
+                "nb_steps": S_, "precision": precision, "gemm_engine": gemm, "cuda_graph": bool(use_graph), "outputs": outputs}
 
     use_graph_any = args.cuda_graph in ("on", "auto")
     use_graph = use_graph_any
@@ -603,6 +665,11 @@ def main():
                                            "single-pass TF32 conditioner GEMMs"),
                         **{k: extra[k] for k in ("value", "ms_per_step", "e2e", "gpu_launches", "roofline", "achieved_tflops_step",
                                                  "algorithmic_gflop_per_step", "nb_steps", "kernel_ms", "cuda_graph")}}
+    if args.dump_outputs:
+        outputs = dict(main_res["outputs"])
+        if extra is not None:
+            outputs.update({"eval." + k: v for k, v in extra["outputs"].items()})
+        dump_outputs(outputs, args.dump_outputs)
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

@@ -336,15 +336,10 @@ def test_umnn_layerwise_rw_and_generic_engines_agree(umnn_engine):
     import os
     import model_vs_oracle as M
     dev_so = os.path.join(os.path.dirname(G._lib.LIB_PATH), "libgnf_sm100_dev.so")
-    if not os.path.isfile(dev_so):
-        pytest.skip("engine override is a development-build knob (build.py --dev): libgnf_sm100_dev.so not built")
+    assert os.path.isfile(dev_so), "engine override is a development-build knob: __graft_entry__.build() builds libgnf_sm100_dev.so"
     devlib = C.CDLL(dev_so)          # the knob is process-global state of THAT library: route the package through it for this test
     product = G._lib._lib
-    try:
-        bound = G._lib._bind(devlib)
-    except AttributeError as err:
-        pytest.skip(f"stale development build (rebuild with build.py --dev): {err}")
-    G._lib._lib = bound
+    G._lib._lib = G._lib._bind(devlib)   # AttributeError: a stale development build (rebuild with build.py --dev)
     umnn_engine("layerwise", "tf32x3")
     model = M.build(M.CONFIGS["cfg4"], "cuda")
     parity.set_modes(model, dict(stoch_gate=False))
