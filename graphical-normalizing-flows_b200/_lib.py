@@ -52,7 +52,6 @@ _PROTOS = {
     "gnf_affine_bwd": ([_P, _P, _I, _P, _P, _P, _P, _P, _P, _P, _I, _I, _P], C.c_int),
     "gnf_normal_ll_fwd": ([_P, _P, _P, _I, _I, _P], C.c_int),
     "gnf_normal_ll_bwd": ([_P, _P, _P, _I, _I, _P], C.c_int),
-    "gnf_logdet_fwd": ([_P, _P, _I, _I, _P], C.c_int),
     "gnf_power_trace_workspace_bytes": ([_I], _SZ),
     "gnf_power_trace_fwd": ([_P, _I, _F, _I, _P, _P, _SZ, _P], C.c_int),
     "gnf_power_trace_bwd": ([_P, _I, _F, _I, _P, _P, _P, _SZ, _P], C.c_int),
@@ -66,11 +65,9 @@ _PROTOS = {
     "gnf_linear_wgrad_tc": ([_P, _I, _P, _I, _P, _I, _I, _I, _I, _I, _P], C.c_int),
     "gnf_linear_wgrad_bias_tc": ([_P, _I, _P, _I, _P, _I, _P, _I, _I, _I, _P], C.c_int),
     "gnf_split_tf32": ([_P, _I, _P, _P, _I, _I, _I, _P], C.c_int),
-    "gnf_linear_tc_ps2": ([_I, _P, _P, _I, _P, _P, _I, _P, _I, _P, _I, _P, _I, _I, _I, _I, _I, _P], C.c_int),
     "gnf_linear_fwd_tc_ps": ([_P, _I, _P, _P, _I, _P, _I, _P, _I, _I, _I, _I, _I, _P], C.c_int),
     "gnf_linear_dgrad_tc_ps": ([_P, _I, _P, _P, _I, _P, _I, _P, _I, _I, _I, _I, _P], C.c_int),
     "gnf_colsum": ([_P, _I, _P, _I, _I, _I, _P], C.c_int),
-    "gnf_relu_mask": ([_P, _I, _P, _I, _I, _I, _P], C.c_int),
     "gnf_pack_rows": ([_P, _P, _P, _P, _I, _I, _P], C.c_int),
     "gnf_unpack_rows": ([_P, _P, _P, _P, _I, _I, _I, _P], C.c_int),
     "gnf_unpack_vec": ([_P, _P, _P, _I, _I, _P], C.c_int),
@@ -132,7 +129,6 @@ _PROTOS = {
     "gnf_reverse_cols": ([_P, _P, _I, _I, _P], C.c_int),
     "gnf_broadcast_rows": ([_P, _P, _I, _I, _I, _I, _P], C.c_int),
     "gnf_counter_add": ([_P, C.c_uint64, _P], C.c_int),
-    "gnf_axpy": ([_F, _P, _P, _SZ, _P], C.c_int),
     "gnf_adam_step": ([C.POINTER(AdamTensorT), _I, _P, _F, _F, _F, _F, _F, _P], C.c_int),
     "gnf_dag_loss_fwd": ([_P, _I, _P, _P, _P, _P, _P, _P, _P], C.c_int),
     "gnf_dag_loss_bwd": ([_P, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P], C.c_int),

@@ -139,16 +139,6 @@ __global__ void nll_loss_bwd_kernel(const float* __restrict__ z, const float* __
     for (size_t b = (size_t)blockIdx.x * blockDim.x + threadIdx.x; b < (size_t)B; b += (size_t)gridDim.x * blockDim.x) glogdet[b] = -s;
 }
 
-__global__ void __launch_bounds__(256) logdet_fwd_kernel(const float* __restrict__ jac, float* __restrict__ logdet, int B, int d) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  for (int b = blockIdx.x * kRowsPerBlock + warp; b < B; b += gridDim.x * kRowsPerBlock) {
-    float acc = 0.f;
-    for (int i = lane; i < d; i += 32) acc += logf(jac[(size_t)b * d + i]);
-    acc = warp_sum(acc);
-    if (lane == 0) logdet[b] = acc;
-  }
-}
-
 __global__ void reverse_cols_kernel(const float* __restrict__ src, float* __restrict__ dst, int B, int d) {
   const size_t n = (size_t)B * d;
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
@@ -168,10 +158,6 @@ __global__ void broadcast_rows_kernel(const float* __restrict__ c, float* __rest
 
 __global__ void counter_add_kernel(unsigned long long* c, unsigned long long inc) {
   if (blockIdx.x == 0 && threadIdx.x == 0) *c += inc;
-}
-
-__global__ void axpy_kernel(float a, const float* __restrict__ x, float* __restrict__ y, size_t n) {
-  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) y[i] = fmaf(a, x[i], y[i]);
 }
 
 static inline int row_blocks(int B) {
@@ -286,13 +272,6 @@ int gnf_nll_loss_bwd(const float* z, const float* g, float* gz, float* glogdet, 
   return check_launch("gnf_nll_loss_bwd");
 }
 
-int gnf_logdet_fwd(const float* jac, float* logdet, int B, int d, gnf_stream_t stream) {
-  if (!jac || !logdet || B < 0 || d <= 0) return fail(GNF_ERR_INVALID, "gnf_logdet_fwd: bad arguments");
-  if (B == 0) return 0;
-  GNF_LAUNCH(logdet_fwd_kernel, row_blocks(B), 256, 0, (cudaStream_t)stream, jac, logdet, B, d);
-  return check_launch("gnf_logdet_fwd");
-}
-
 int gnf_reverse_cols(const float* src, float* dst, int B, int d, gnf_stream_t stream) {
   if (!src || !dst || B < 0 || d <= 0) return fail(GNF_ERR_INVALID, "gnf_reverse_cols: bad arguments");
   if (B == 0) return 0;
@@ -326,13 +305,6 @@ int gnf_dag_loss_bwd(const float* A, int d, const float* t, const float* lambd, 
   if (!A || !t || !lambd || !c || !dag_const || !l1_weight || !gout || !dA || !dt || d <= 0) return fail(GNF_ERR_INVALID, "gnf_dag_loss_bwd: bad arguments");
   GNF_LAUNCH(dag_loss_bwd_kernel, flat_blocks((size_t)d * d), 256, 0, (cudaStream_t)stream, A, d * d, t, lambd, c, dag_const, l1_weight, gout, dA, dt);
   return check_launch("gnf_dag_loss_bwd");
-}
-
-int gnf_axpy(float a, const float* x, float* y, size_t n, gnf_stream_t stream) {
-  if (!x || !y) return fail(GNF_ERR_INVALID, "gnf_axpy: bad arguments");
-  if (n == 0) return 0;
-  GNF_LAUNCH(axpy_kernel, flat_blocks(n), 256, 0, (cudaStream_t)stream, a, x, y, n);
-  return check_launch("gnf_axpy");
 }
 
 }  // extern "C"

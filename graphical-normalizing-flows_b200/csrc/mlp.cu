@@ -621,14 +621,6 @@ __global__ void colsum_kernel(const float* __restrict__ Y, float* __restrict__ o
   }
 }
 
-__global__ void relu_mask_kernel(float* dY, int lddy, const float* __restrict__ act, int ldact, int M, int N) {
-  const size_t n = (size_t)M * N;
-  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
-    const size_t m = i / N, c = i % N;
-    if (!(act[m * ldact + c] > 0.f)) dY[m * lddy + c] = 0.f;
-  }
-}
-
 __global__ void pack_rows_kernel(const float* __restrict__ W, const float* __restrict__ mask, const int32_t* __restrict__ perm, float* __restrict__ out, int R, int K) {
   const size_t n = (size_t)R * K;
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
@@ -819,13 +811,6 @@ int gnf_colsum(const float* Y, int ldy, float* out, int M, int N, int period, gn
   const int q_per = ceil_div(Q, qsplit);
   GNF_LAUNCH(colsum_kernel, dim3(cblocks, ceil_div(Q, q_per)), 256, 0, s, Y, out, Q, C, ldy, N, (size_t)period * ldy, q_per);
   return check_launch("gnf_colsum");
-}
-
-int gnf_relu_mask(float* dY, int lddy, const float* act, int ldact, int M, int N, gnf_stream_t stream) {
-  if (!dY || !act || M < 0 || N <= 0) return fail(GNF_ERR_INVALID, "gnf_relu_mask: bad arguments");
-  if (M == 0) return 0;
-  GNF_LAUNCH(relu_mask_kernel, ew_blocks((size_t)M * N), 256, 0, (cudaStream_t)stream, dY, lddy, act, ldact, M, N);
-  return check_launch("gnf_relu_mask");
 }
 
 int gnf_pack_rows(const float* W, const float* mask, const int32_t* perm, float* out, int R, int K, gnf_stream_t stream) {

@@ -173,14 +173,12 @@ __device__ __forceinline__ void trace_stamp(long long* trace, int role, long lon
 }
 
 __global__ void __launch_bounds__(kGemmThreads) tc_gemm_kernel(TcGemmParams p, int vecA, int vecB, const __grid_constant__ CUtensorMap tmA,
-                                                               const __grid_constant__ CUtensorMap tmB, const __grid_constant__ CUtensorMap tmBlo,
-                                                               const __grid_constant__ CUtensorMap tmAlo) {
+                                                               const __grid_constant__ CUtensorMap tmB, const __grid_constant__ CUtensorMap tmBlo) {
   using namespace tc;
   GNF_SMEM(char, smem);
   const int BN = p.BN;
   const bool split = p.passes == 3;
   const bool presplit = split && p.B_lo != nullptr;      // B arrives as separate hi / lo tiles (only with TMA)
-  const bool presplitA = presplit && p.A_lo != nullptr;  // so does A: nothing left to split, the MMA warp consumes the landed tiles
   const uint32_t a_bytes = kGemmBM * 128u, b_bytes = (uint32_t)BN * 128u;
   const uint32_t stage_bytes = (a_bytes + b_bytes) * (split ? 2u : 1u);
   // stage layout: [A_hi][B_hi]([A_lo][B_lo]); then the epilogue transpose blocks; then the barriers
@@ -222,14 +220,9 @@ __global__ void __launch_bounds__(kGemmThreads) tc_gemm_kernel(TcGemmParams p, i
           mbar_wait(&empty[s], (uint32_t)(((it / p.stages) & 1) ^ 1));
           char* st = smem + (size_t)s * stage_bytes;
           if (isA) {
-            mbar_expect_tx(&landed[s], presplitA ? 2u * a_bytes : a_bytes);
+            mbar_expect_tx(&landed[s], a_bytes);
             if (p.a_src == TCG_SRC_K) tma_load_2d(st, &tmA, k0, tm * kGemmBM, &landed[s]);
             else for (int sl = 0; sl < kGemmBM / 32; ++sl) tma_load_2d(st + sl * 4096, &tmA, tm * kGemmBM + 32 * sl, k0, &landed[s]);
-            if (presplitA) {
-              char* lo = st + a_bytes + b_bytes;
-              if (p.a_src == TCG_SRC_K) tma_load_2d(lo, &tmAlo, k0, tm * kGemmBM, &landed[s]);
-              else for (int sl = 0; sl < kGemmBM / 32; ++sl) tma_load_2d(lo + sl * 4096, &tmAlo, tm * kGemmBM + 32 * sl, k0, &landed[s]);
-            }
             trace_stamp(p.trace, 0, it);
           } else {
             mbar_expect_tx(&landed[s], presplit ? 2u * b_bytes : b_bytes);
@@ -260,7 +253,7 @@ __global__ void __launch_bounds__(kGemmThreads) tc_gemm_kernel(TcGemmParams p, i
       if (lane == 0) mbar_arrive(&full[s]);
     };
     if (p.use_tma) {
-      if (split && !presplitA) {                         // single-pass TF32 / fully pre-split: the MMA warp consumes the landed tiles directly
+      if (split) {                                       // 3xTF32 only: single-pass TF32 MMAs consume the landed tiles directly
         for (long long w = blockIdx.x; w < total; w += gridDim.x) {
           const int sp = (int)(w / ((long long)tiles_m * tiles_n));
           const int kbeg = sp * p.k_per_split, kend = min(p.K, kbeg + p.k_per_split);
@@ -304,7 +297,7 @@ __global__ void __launch_bounds__(kGemmThreads) tc_gemm_kernel(TcGemmParams p, i
       // per k-step (8 k) descriptor advance: K-major: 32 bytes inside the swizzle atom; MN-major: 8 tile rows = 1024 bytes
       const uint32_t a_step = (p.a_src == TCG_SRC_K) ? 2u : 64u, b_step = (p.b_src == TCG_SRC_K) ? 2u : 64u;
       const bool a_mn = p.a_src == TCG_SRC_MN, b_mn = p.b_src == TCG_SRC_MN;
-      uint64_t* ready = (p.use_tma && (!split || presplitA)) ? landed : full;
+      uint64_t* ready = (p.use_tma && !split) ? landed : full;
       long long it = 0;
       int gcount = 0;                                    // accumulator groups issued so far (buffer = gcount & 1)
       for (long long w = blockIdx.x; w < total; w += gridDim.x) {
@@ -647,8 +640,7 @@ static int g_tc_gemm_fold2 = 2;     // ... of engine v2 (forward / dgrad with pr
                                     // gradients of A / W1 at cfg5 sit on ReLU-flip noise of that size (profiles/r02p_cfg5_grad_accuracy*.txt).
 static bool g_tc_gemm_fold_forced = false;   // dev build: gnf_tc_gemm_set_fold overrides both rules
 static bool g_tc_gemm_tma = true;   // measurement switch (gnf_tc_gemm_set_tma): 0 forces the cp.async staging path
-static int g_tc_gemm_v2 = 1;        // measurement switch (gnf_tc_gemm_set_v2, dev build): 0 keeps forward / dgrad on the engine above,
-                                    // 1 = two partial accumulators + four A buffers, 2 = three partials + two A buffers
+static int g_tc_gemm_v2 = 1;        // measurement switch (gnf_tc_gemm_set_v2, dev build): 0 keeps forward / dgrad on the engine above
 
 // hi = rn_tf32(W), lo = rn_tf32(W - hi), both [N][ld] with zero padding columns (ld >= K)
 __global__ void split_tf32_kernel(const float* __restrict__ W, long long ldw, float* __restrict__ hi, float* __restrict__ lo, int ld, int N, int K) {
@@ -669,7 +661,7 @@ __global__ void split_tf32_kernel(const float* __restrict__ W, long long ldw, fl
 // tile into hi / lo tiles in shared memory -- and the 16-column transposing epilogue takes 24 k clocks per tile.  Here:
 //   * the activation operand never exists as an MMA tile in shared memory: four A-writer warps (thread = tile row = TMEM
 //     lane) read their row of the TMA-landed raw tile (conflict-free through the 128B swizzle), split it in registers and
-//     write A_hi / A_lo into a two-deep TMEM ring (tcgen05.st); the MMAs are TS form, B = the pre-split weight tiles;
+//     write A_hi / A_lo into a four-deep TMEM ring (tcgen05.st); the MMAs are TS form, B = the pre-split weight tiles;
 //   * a stage is 48 KB (raw A + B_hi + B_lo) instead of 64 KB: four stages in flight;
 //   * same accumulation discipline as above (the tensor core truncates its accumulator after every MMA, one-sided): two
 //     partial accumulators in TMEM, folded every `fold` k-chunks into a round-to-nearest running sum that EIGHT epilogue
@@ -683,10 +675,7 @@ constexpr int kG2BN = 128, kG2Stages = 4, kG2Threads = 14 * 32;   // 8 epilogue 
 constexpr uint32_t kG2TileBytes = 128u * 128u;                    // one 128-row x 32-k fp32 tile
 constexpr uint32_t kG2StageBytes = 3u * kG2TileBytes;             // raw A, B_hi, B_lo
 constexpr int kG2EpiStageFloats = 32 * 32;
-constexpr int kG2MaxRing = 4, kG2MaxParts = 3;
-
-// kParts partial accumulators of 128 TMEM columns, then kRing A buffers of (hi 32 + lo 32) columns: (2, 4) or (3, 2) fill 512.
-template <int kParts, int kRing>
+constexpr int kG2Parts = 2, kG2Ring = 4;   // partial accumulators of 128 TMEM columns, then A buffers of (hi 32 + lo 32) columns
 
 __global__ void __launch_bounds__(kG2Threads, 1) tc_gemm2_kernel(TcGemmParams p, const __grid_constant__ CUtensorMap tmA,
                                                                  const __grid_constant__ CUtensorMap tmB, const __grid_constant__ CUtensorMap tmBlo) {
@@ -696,20 +685,20 @@ __global__ void __launch_bounds__(kG2Threads, 1) tc_gemm2_kernel(TcGemmParams p,
   uint64_t* bars = reinterpret_cast<uint64_t*>(epi_stage + 8 * kG2EpiStageFloats);
   uint64_t* landed = bars;                     // [stages] TMA -> A-writers / MMA (transaction bytes)
   uint64_t* empty = landed + kG2Stages;        // [stages] MMA -> producer (tcgen05.commit)
-  constexpr uint32_t kG2ColA = 128u * kParts;
-  static_assert(kG2ColA + 64u * kRing <= 512u && kParts <= kG2MaxParts && kRing <= kG2MaxRing, "TMEM budget");
-  uint64_t* a_full = empty + kG2Stages;        // [kRing] A-writers -> MMA (one arrive per writer warp)
-  uint64_t* a_empty = a_full + kG2MaxRing;     // [kRing] MMA -> A-writers (tcgen05.commit)
-  uint64_t* tfull = a_empty + kG2MaxRing;      // [kParts] MMA -> epilogue
-  uint64_t* tempty = tfull + kG2MaxParts;      // [kParts] epilogue -> MMA (one arrive per epilogue warp)
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tempty + kG2MaxParts);
+  constexpr uint32_t kG2ColA = 128u * kG2Parts;
+  static_assert(kG2ColA + 64u * kG2Ring <= 512u, "TMEM budget");
+  uint64_t* a_full = empty + kG2Stages;        // [kG2Ring] A-writers -> MMA (one arrive per writer warp)
+  uint64_t* a_empty = a_full + kG2Ring;        // [kG2Ring] MMA -> A-writers (tcgen05.commit)
+  uint64_t* tfull = a_empty + kG2Ring;         // [kG2Parts] MMA -> epilogue
+  uint64_t* tempty = tfull + kG2Parts;         // [kG2Parts] epilogue -> MMA (one arrive per epilogue warp)
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tempty + kG2Parts);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
 
   if (warp == 0) tmem_alloc(tmem_slot, 512);
   if (tid == 32) {
     for (int s = 0; s < kG2Stages; ++s) { mbar_init(&landed[s], 1); mbar_init(&empty[s], 1); }
-    for (int b = 0; b < kRing; ++b) { mbar_init(&a_full[b], 4); mbar_init(&a_empty[b], 1); }
-    for (int b = 0; b < kParts; ++b) { mbar_init(&tfull[b], 1); mbar_init(&tempty[b], 8); }
+    for (int b = 0; b < kG2Ring; ++b) { mbar_init(&a_full[b], 4); mbar_init(&a_empty[b], 1); }
+    for (int b = 0; b < kG2Parts; ++b) { mbar_init(&tfull[b], 1); mbar_init(&tempty[b], 8); }
     fence_mbar_init();
   }
   fence_before_sync();
@@ -756,15 +745,15 @@ __global__ void __launch_bounds__(kG2Threads, 1) tc_gemm2_kernel(TcGemmParams p,
     int it = 0, gcount = 0;
     for (int w = blockIdx.x; w < total; w += gridDim.x) {
       for (int c0 = 0; c0 < nchunks; c0 += fold, ++gcount) {
-        const int acc = gcount % kParts;
-        mbar_wait(&tempty[acc], (uint32_t)(((gcount / kParts) & 1) ^ 1));
+        const int acc = gcount % kG2Parts;
+        mbar_wait(&tempty[acc], (uint32_t)(((gcount / kG2Parts) & 1) ^ 1));
         fence_after_sync();
         const uint32_t d_tmem = tmem_base + (uint32_t)acc * kG2BN;
         const int c1 = (c0 + fold < nchunks) ? c0 + fold : nchunks;
         uint32_t first = 0u;
         for (int c = c0; c < c1; ++c, ++it) {
-          const int s = it % kG2Stages, b = it % kRing;
-          mbar_wait(&a_full[b], (uint32_t)((it / kRing) & 1));
+          const int s = it % kG2Stages, b = it % kG2Ring;
+          mbar_wait(&a_full[b], (uint32_t)((it / kG2Ring) & 1));
           mbar_wait(&landed[s], (uint32_t)((it / kG2Stages) & 1));
           fence_after_sync();
           if (lane == 0) trace_stamp(p.trace, 3, it);
@@ -797,7 +786,7 @@ __global__ void __launch_bounds__(kG2Threads, 1) tc_gemm2_kernel(TcGemmParams p,
     int it = 0;
     for (int w = blockIdx.x; w < total; w += gridDim.x) {
       for (int c = 0; c < nchunks; ++c, ++it) {
-        const int s = it % kG2Stages, b = it % kRing;
+        const int s = it % kG2Stages, b = it % kG2Ring;
         mbar_wait(&landed[s], (uint32_t)((it / kG2Stages) & 1));
         if (tid == 256) trace_stamp(p.trace, 1, it);
         const char* rp = smem + (size_t)s * kG2StageBytes + row * 128;
@@ -813,7 +802,7 @@ __global__ void __launch_bounds__(kG2Threads, 1) tc_gemm2_kernel(TcGemmParams p,
             lo[4 * j + k] = __float_as_uint(__uint_as_float(e[k]) - __uint_as_float(h)) + 0x1000u;   // the tensor core drops the low bits
           }
         }
-        mbar_wait(&a_empty[b], (uint32_t)(((it / kRing) & 1) ^ 1));
+        mbar_wait(&a_empty[b], (uint32_t)(((it / kG2Ring) & 1) ^ 1));
         fence_after_sync();
         const uint32_t ta = tmem_base + lane_sel + kG2ColA + (uint32_t)b * 64u;
         tmem_st32p(ta, hi);
@@ -867,8 +856,8 @@ __global__ void __launch_bounds__(kG2Threads, 1) tc_gemm2_kernel(TcGemmParams p,
         }
       }
       for (int g = 0; g < ngroups; ++g, ++gcount) {
-        const int acc = gcount % kParts;
-        mbar_wait(&tfull[acc], (uint32_t)((gcount / kParts) & 1));
+        const int acc = gcount % kG2Parts;
+        mbar_wait(&tfull[acc], (uint32_t)((gcount / kG2Parts) & 1));
         fence_after_sync();
         if (tid == 0) trace_stamp(p.trace, 5, gcount);
         const uint32_t part = tmem_base + lane_sel + (uint32_t)acc * kG2BN + (uint32_t)ch;
@@ -965,7 +954,7 @@ __global__ void __launch_bounds__(kG2Threads, 1) tc_gemm2_kernel(TcGemmParams p,
 }
 
 static bool g2_eligible(const TcGemmParams& p) {
-  if (p.passes != 3 || !p.B_lo || p.A_lo || p.a_src != TCG_SRC_K || p.epi == TCG_EPI_ATOMIC || p.bits_out || p.mask_bits) return false;
+  if (p.passes != 3 || !p.B_lo || p.a_src != TCG_SRC_K || p.epi == TCG_EPI_ATOMIC || p.bits_out || p.mask_bits) return false;
   if (p.epi == TCG_EPI_BIAS_ACT && p.bias && (reinterpret_cast<uintptr_t>(p.bias) & 15) != 0) return false;
   if (p.epi == TCG_EPI_BIAS_ACT && p.bias && p.bias_period > 1 && ((p.bias_ld % 4) != 0 || p.bias_ld < (p.N + 3) / 4 * 4)) return false;   // 16-byte pieces inside the (padded) table row
   if (p.epi == TCG_EPI_MASK && p.act && ((reinterpret_cast<uintptr_t>(p.act) & 15) != 0 || (p.ldact % 4) != 0)) return false;
@@ -1228,7 +1217,7 @@ __global__ void __launch_bounds__(kW2Threads, 1) tc_wgrad2_kernel(TcGemmParams p
 }
 
 static bool w2_eligible(const TcGemmParams& p) {
-  if (p.passes != 3 || p.epi != TCG_EPI_ATOMIC || p.a_src != TCG_SRC_MN || p.b_src != TCG_SRC_MN || p.A_lo || p.B_lo) return false;
+  if (p.passes != 3 || p.epi != TCG_EPI_ATOMIC || p.a_src != TCG_SRC_MN || p.b_src != TCG_SRC_MN || p.B_lo) return false;
   if (p.M < 256 || p.K < 2048) return false;               // small problems: the planned tiling of the first engine
   return p.N >= 256 || (p.N >= 32 && p.N <= 64);           // ... or ONE narrow tile column (layer 1 of a narrow DAG flow against the gate plane)
 }
@@ -1274,19 +1263,15 @@ int launch_tc_gemm(TcGemmParams p, cudaStream_t s) {
   p.c_vec = ((reinterpret_cast<uintptr_t>(p.C) & 15) == 0 && (p.ldc % 4) == 0) ? 1 : 0;
   p.act_vec = (p.act && (reinterpret_cast<uintptr_t>(p.act) & 15) == 0 && (p.ldact % 4) == 0) ? 1 : 0;
   p.bias_vec = (p.bias && (reinterpret_cast<uintptr_t>(p.bias) & 15) == 0 && (p.bias_ld % 4) == 0) ? 1 : 0;
-  CUtensorMap tmA, tmB, tmBlo, tmAlo;
+  CUtensorMap tmA, tmB, tmBlo;
   memset(&tmA, 0, sizeof(tmA));
   memset(&tmB, 0, sizeof(tmB));
   memset(&tmBlo, 0, sizeof(tmBlo));
-  memset(&tmAlo, 0, sizeof(tmAlo));
   p.use_tma = (g_tc_gemm_tma && make_operand_map(&tmA, p.A, p.lda, p.a_src, p.M, p.K, kGemmBM) &&
                make_operand_map(&tmB, p.B, p.ldb, p.b_src, p.N, p.K, p.BN)) ? 1 : 0;
   if (p.passes != 3) p.B_lo = nullptr;
   if (p.B_lo && !(p.use_tma && make_operand_map(&tmBlo, p.B_lo, p.ldb, p.b_src, p.N, p.K, p.BN)))
     return fail(GNF_ERR_UNSUPPORTED, "tensor-core GEMM: pre-split weights need TMA-loadable operands (16-byte aligned rows)");
-  if (!p.B_lo) p.A_lo = nullptr;
-  if (p.A_lo && !make_operand_map(&tmAlo, p.A_lo, p.lda, p.a_src, p.M, p.K, kGemmBM))
-    return fail(GNF_ERR_UNSUPPORTED, "tensor-core GEMM: pre-split activations need TMA-loadable operands (16-byte aligned rows)");
   if (g_tc_gemm_v2 && p.use_tma && w2_eligible(p)) {
     // engine v2, weight gradient: BN = 128, its own split plan (MN-major maps have 32 x 32 boxes whatever the tile width)
     p.BN = kG2BN;
@@ -1315,18 +1300,11 @@ int launch_tc_gemm(TcGemmParams p, cudaStream_t s) {
     p.fold = (!g_tc_gemm_fold_forced && p.epi == TCG_EPI_BIAS_ACT && p.bias && p.bias_period > 1) ? 1 : g_tc_gemm_fold2;
     p.trace = g_tc_gemm_trace;
     const size_t smem2 = (size_t)kG2Stages * kG2StageBytes + 8 * kG2EpiStageFloats * sizeof(float) +
-                         (2 * kG2Stages + 2 * kG2MaxRing + 2 * kG2MaxParts) * sizeof(uint64_t) + 16;
+                         (2 * kG2Stages + 2 * kG2Ring + 2 * kG2Parts) * sizeof(uint64_t) + 16;
     const int total2 = ((p.M + kGemmBM - 1) / kGemmBM) * ((p.N + kG2BN - 1) / kG2BN);
     const int grid2 = total2 < kNumSMs ? total2 : kNumSMs;
-#ifdef GNF_DEVTOOLS
-    if (g_tc_gemm_v2 == 2) {                     // measured equal to the default below at every fold interval (profiles/r02q_gemm2_fold_variants.txt)
-      cudaFuncSetAttribute(tc_gemm2_kernel<3, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2);
-      GNF_LAUNCH_PDL((tc_gemm2_kernel<3, 2>), grid2, kG2Threads, smem2, s, p, tmA, tmB, tmBlo);
-      return 0;
-    }
-#endif
-    cudaFuncSetAttribute(tc_gemm2_kernel<2, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2);
-    GNF_LAUNCH_PDL((tc_gemm2_kernel<2, 4>), grid2, kG2Threads, smem2, s, p, tmA, tmB, tmBlo);
+    cudaFuncSetAttribute(tc_gemm2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2);
+    GNF_LAUNCH_PDL(tc_gemm2_kernel, grid2, kG2Threads, smem2, s, p, tmA, tmB, tmBlo);
     return 0;
   }
   p.trace = g_tc_gemm_trace;
@@ -1335,7 +1313,7 @@ int launch_tc_gemm(TcGemmParams p, cudaStream_t s) {
   // per launch: the attribute is per DEVICE, a process-wide "done" flag breaks the second GPU of a process (and is racy)
   cudaFuncSetAttribute(tc_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBudget);
   const int grid = (int)(total < kNumSMs ? total : kNumSMs);
-  GNF_LAUNCH_PDL(tc_gemm_kernel, grid, kGemmThreads, smem, s, p, vec_width(p.A, p.lda), vec_width(p.B, p.ldb), tmA, tmB, tmBlo, tmAlo);
+  GNF_LAUNCH_PDL(tc_gemm_kernel, grid, kGemmThreads, smem, s, p, vec_width(p.A, p.lda), vec_width(p.B, p.ldb), tmA, tmB, tmBlo);
   return 0;
 }
 
@@ -1437,39 +1415,6 @@ int gnf_linear_dgrad_tc_ps(const float* dY, int lddy, const float* W_hi, const f
 #endif
 }
 
-int gnf_linear_tc_ps2(int op, const float* A_hi, const float* A_lo, int lda, const float* B_hi, const float* B_lo, int ldb, const float* bias,
-                      int bias_period, const float* act, int ldact, float* C, int ldc, int M, int N, int K, int relu, gnf_stream_t stream) {
-#ifdef GNF_EMU
-  return gnf::fail(GNF_ERR_UNSUPPORTED, "tensor-core kernels have no host-simulator flavour");
-#else
-  if (!A_hi || !A_lo || !B_hi || !B_lo || !C || M < 0 || N <= 0 || K <= 0 || op < 0 || op > 2) return fail(GNF_ERR_INVALID, "gnf_linear_tc_ps2: bad arguments");
-  cudaStream_t s = (cudaStream_t)stream;
-  TcGemmParams p = {};
-  p.passes = 3;
-  if (op == 0) {            // forward: Y[M,N] = act(X[M,K] W[N,K]^T + b);  A = X, B = W
-    p.A = A_hi; p.A_lo = A_lo; p.lda = lda; p.a_src = TCG_SRC_K;
-    p.B = B_hi; p.B_lo = B_lo; p.ldb = ldb; p.b_src = TCG_SRC_K;
-    p.M = M; p.N = N; p.K = K;
-    p.epi = TCG_EPI_BIAS_ACT; p.C = C; p.ldc = ldc; p.bias = bias; p.bias_ld = N; p.bias_period = bias_period < 1 ? 1 : bias_period; p.relu = relu;
-  } else if (op == 1) {     // dgrad: dX[M,K] = (dY[M,N] W[N,K]) o relu'(act);  A = dY, B = W (MN-major)
-    p.A = A_hi; p.A_lo = A_lo; p.lda = lda; p.a_src = TCG_SRC_K;
-    p.B = B_hi; p.B_lo = B_lo; p.ldb = ldb; p.b_src = TCG_SRC_MN;
-    p.M = M; p.N = K; p.K = N;
-    p.epi = TCG_EPI_MASK; p.C = C; p.ldc = ldc; p.act = act; p.ldact = ldact;
-  } else {                  // wgrad: dW[N,K] = dY[M,N]^T X[M,K];  A = dY (MN-major), B = X (MN-major), split-K atomics into zeroed dW
-    if (ldc == K) cudaMemsetAsync(C, 0, (size_t)N * K * sizeof(float), s);
-    else for (int n = 0; n < N; ++n) cudaMemsetAsync(C + (size_t)n * ldc, 0, (size_t)K * sizeof(float), s);
-    if (M == 0) return check_launch("gnf_linear_tc_ps2");
-    p.A = A_hi; p.A_lo = A_lo; p.lda = lda; p.a_src = TCG_SRC_MN;
-    p.B = B_hi; p.B_lo = B_lo; p.ldb = ldb; p.b_src = TCG_SRC_MN;
-    p.M = N; p.N = K; p.K = M;
-    p.epi = TCG_EPI_ATOMIC; p.C = C; p.ldc = ldc;
-  }
-  if (int e = launch_tc_gemm(p, s)) return e;
-  return check_launch("gnf_linear_tc_ps2");
-#endif
-}
-
 #ifdef GNF_DEVTOOLS
 int gnf_tc_gemm_set_trace(long long* buf) {
 #ifdef GNF_EMU
@@ -1525,6 +1470,7 @@ int gnf_tc_gemm_plan(int M, int N, int K, int passes, int wgrad, int* bn, int* s
 
 #ifdef GNF_DEVTOOLS
 int gnf_tc_gemm_set_v2(int enable) {
+  if (enable != 0 && enable != 1) return gnf::fail(GNF_ERR_INVALID, "gnf_tc_gemm_set_v2: 0 (first engine) or 1 (engine v2)");
 #ifndef GNF_EMU
   gnf::g_tc_gemm_v2 = enable;
 #else

@@ -11,7 +11,6 @@ enum { TCG_SRC_K = 0, TCG_SRC_MN = 1 };  // global memory contiguous along the r
 struct TcGemmParams {
   // C[m, n] = sum_k A(m, k) * B(n, k);  A: Mrows x Kred,  B: Ncols x Kred
   const float* A; long long lda; int a_src;    // TCG_SRC_K: A(m,k) = A[m*lda + k];  TCG_SRC_MN: A(m,k) = A[k*lda + m]
-  const float* A_lo;                           // 3xTF32 only, nullable: pre-split A, as B_lo below (needs B_lo as well)
   const float* B; long long ldb; int b_src;    // same convention with n in place of m
   const float* B_lo;                           // 3xTF32 only, nullable: B is already rn_tf32(b) and B_lo = rn_tf32(b - B) (same layout):
                                                // both are TMA-loaded and the stagers skip the B split (weights: split once per call)

@@ -27,7 +27,7 @@ def _device_noise_counters(model, dev):
 def model_graph_state(model):
     """Host-side state a captured step froze (ADVICE r1): conditioner flags / exponents / buffer addresses
     (DAGConditioner.graph_state), quadrature steps and precision of the normalizers, and the engine switches."""
-    st = [ops._GEMM_MODE, ops.UMNN_ENGINE, ops.UMNN_FWD_FUSED_TC3, ops.UMNN_BWD_FUSED_TC3]
+    st = [ops._GEMM_MODE, ops.UMNN_ENGINE, ops.UMNN_FWD_FUSED_TC3]
     for c in model.getConditioners():
         st.append(c.graph_state() if hasattr(c, "graph_state") else None)
     for n in model.getNormalizers():

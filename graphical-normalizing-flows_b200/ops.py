@@ -65,10 +65,10 @@ def _note_flops(name, flops, shape=None):
         _SHAPES.setdefault(name, []).append(shape)
 
 
-def tc_kernel_name(op, M, N, K, passes=3, presplit=True):
+def tc_kernel_name(op, M, N, K, passes=3):
     """Which kernel of the tcgen05 GEMM engine a layer call of this shape launches (mirrors g2_eligible / w2_eligible in
     csrc/tc_gemm.cu for TMA-loadable operands): op 'fwd' / 'dgrad' (M rows, N out-features, K in-features) or 'wgrad'."""
-    if passes == 3 and presplit:
+    if passes == 3:
         if op == "wgrad":
             return "tc_wgrad2_kernel" if (N >= 256 and (K >= 256 or 32 <= K <= 64) and M >= 2048) else "tc_gemm_kernel"
         n, k = (N, K) if op == "fwd" else (K, N)
@@ -409,14 +409,14 @@ def _tma_weight(W):
 
 
 SPLITK_SKINNY = True         # skinny layers with a long reduction (630 -> 30) on the FFMA engine: deterministic split-K (gnf_linear_fwd_splitk)
-PRESPLIT_WEIGHTS = True      # 3xTF32: split the weights once per call (gnf_split_tf32) instead of per tile in shared memory
 
 
 _SPLIT_CACHE = {}
 
 
 def _split_weight(W):
-    """(W_hi, W_lo) with rows padded to 4 floats, for the *_tc_ps entry points.  The forward's split is reused by the same
+    """(W_hi, W_lo) with rows padded to 4 floats, for the *_tc_ps entry points: in 3xTF32 the weights are split once per call
+    (gnf_split_tf32) instead of per tile in shared memory.  The forward's split is reused by the same
     step's dgrad: keyed by storage and version (optimizers update in place, which bumps the version), and by the stream
     capture state so that a captured step never refers to tensors made outside its graph."""
     key = (W.data_ptr(), W._version, tuple(W.shape), torch.cuda.is_current_stream_capturing() if W.is_cuda else False)
@@ -438,34 +438,8 @@ def _tma_ok(t, ld):
     return t.data_ptr() % 16 == 0 and ld % 4 == 0
 
 
-# ... and optionally the activation operands too (one elementwise pass each, shared by the GEMMs that read them).  Measured on
-# cfg4 (profiles/r01zq): with nothing left to split in shared memory the k-chunk cadence does not move (72 us forward either way) --
-# four TMA tiles per chunk (72 KB) put the kernel on the L2 -> SM bandwidth instead (29 B/clk/SM = 8.4 TB/s over the chip) -- and
-# only wgrad gains (98 -> 77 us), which the two extra passes eat.  Off by default; kept (and tested) for multicast clusters.
-PRESPLIT_ACTS = False
-PRESPLIT_ACTS_MIN_K = 256    # short reductions do not amortise the extra pass
-
-
-def _split_mat(X, M, K, ldx):
-    """TF32 (hi, lo) copies of the [M, K] matrix at X (row stride ldx), rows padded to 4 floats."""
-    hi = torch.empty(M, _pad4(K), device=X.device, dtype=X.dtype)
-    lo = torch.empty_like(hi)
-    _call("gnf_split_tf32", ptr(X), ldx, ptr(hi), ptr(lo), hi.stride(0), M, K, stream_ptr())
-    _count()
-    return hi, lo
-
-
-def _ps2(op, A, B, ldab, bias, bias_period, act, C, ldc, M, N, K, relu, name):
-    """gnf_linear_tc_ps2 with both operands pre-split; A, B = (hi, lo) pairs."""
-    _note_flops(name, 2. * M * N * K, (M, N, K))
-    _TIMES_ALIAS["gnf_linear_tc_ps2"] = name
-    _call("gnf_linear_tc_ps2", op, ptr(A[0]), ptr(A[1]), ldab[0], ptr(B[0]), ptr(B[1]), ldab[1], ptr(bias), bias_period,
-          ptr(act), (act.stride(0) if act is not None else 0), ptr(C), ldc, M, N, K, int(relu), stream_ptr())
-
-
-def linear_fwd(X, W, bias, relu, bias_period=1, out=None, ldy=None, K=None, ldx=None, x_split=None, want_split=False):
-    """Y = act(X[:, :K] @ W^T + bias).  X may be a row-strided view described by (ldx, K).
-    x_split: (hi, lo) of X if the caller has them; want_split: also return the pair this call used (or None)."""
+def linear_fwd(X, W, bias, relu, bias_period=1, out=None, ldy=None, K=None, ldx=None):
+    """Y = act(X[:, :K] @ W^T + bias).  X may be a row-strided view described by (ldx, K)."""
     M = X.shape[0]
     N = W.shape[0]
     K = W.shape[1] if K is None else K
@@ -474,12 +448,7 @@ def linear_fwd(X, W, bias, relu, bias_period=1, out=None, ldy=None, K=None, ldx=
         out = _rows(M, N, X)
         ldy = out.stride(0)
     passes = _gemm_passes(M, N, K)
-    used = None
-    if passes == 3 and PRESPLIT_WEIGHTS and PRESPLIT_ACTS and K == W.shape[1] and K >= PRESPLIT_ACTS_MIN_K and M > 0:
-        used = x_split if x_split is not None else _split_mat(X, M, K, ldx)
-        wh, wl = _split_weight(W)
-        _ps2(0, used, (wh, wl), (used[0].stride(0), wh.stride(0)), bias, bias_period, None, out, ldy, M, N, K, relu, "gnf_linear_fwd_tc")
-    elif passes == 3 and PRESPLIT_WEIGHTS and _tma_ok(X, ldx) and K == W.shape[1]:
+    if passes == 3 and _tma_ok(X, ldx) and K == W.shape[1]:
         hi, lo = _split_weight(W)
         _note_flops("gnf_linear_fwd_tc", 2. * M * N * K, (M, N, K))
         _TIMES_ALIAS["gnf_linear_fwd_tc_ps"] = "gnf_linear_fwd_tc"
@@ -502,19 +471,16 @@ def linear_fwd(X, W, bias, relu, bias_period=1, out=None, ldy=None, K=None, ldx=
             _call("gnf_linear_fwd", ptr(X), ldx, ptr(W), W.stride(0), ptr(bias), bias_period, ptr(out), ldy, M, N, K, int(relu),
                   stream_ptr())
     _count()
-    return (out, used) if want_split else out
+    return out
 
 
-def linear_dgrad(dY, lddy, W, act, M, out=None, lddx=None, dy_split=None):
+def linear_dgrad(dY, lddy, W, act, M, out=None, lddx=None):
     N, K = W.shape
     if out is None:
         out = _rows(M, K, dY)
         lddx = out.stride(0)
     passes = _gemm_passes(M, N, K)
-    if passes == 3 and PRESPLIT_WEIGHTS and PRESPLIT_ACTS and dy_split is not None:
-        wh, wl = _split_weight(W)
-        _ps2(1, dy_split, (wh, wl), (dy_split[0].stride(0), wh.stride(0)), None, 1, act, out, lddx, M, N, K, 0, "gnf_linear_dgrad_tc")
-    elif passes == 3 and PRESPLIT_WEIGHTS and _tma_ok(dY, lddy):
+    if passes == 3 and _tma_ok(dY, lddy):
         hi, lo = _split_weight(W)
         _note_flops("gnf_linear_dgrad_tc", 2. * M * N * K, (M, N, K))
         _TIMES_ALIAS["gnf_linear_dgrad_tc_ps"] = "gnf_linear_dgrad_tc"
@@ -532,14 +498,12 @@ def linear_dgrad(dY, lddy, W, act, M, out=None, lddx=None, dy_split=None):
     return out
 
 
-def linear_wgrad(dY, lddy, X, ldx, M, N, K, dy_split=None, x_split=None, out=None, lddw=None):
+def linear_wgrad(dY, lddy, X, ldx, M, N, K, out=None, lddw=None):
     """dW[n, k] = sum_m dY[m, n] X[m, k]; `out` / `lddw`: write into the first K columns of a wider [N, lddw] matrix."""
     dW = torch.empty(N, K, device=dY.device, dtype=dY.dtype) if out is None else out
     lddw = K if out is None else lddw
     passes = _gemm_passes(M, N, K, "wgrad")
-    if passes == 3 and PRESPLIT_ACTS and dy_split is not None and x_split is not None:
-        _ps2(2, dy_split, x_split, (dy_split[0].stride(0), x_split[0].stride(0)), None, 1, None, dW, lddw, M, N, K, 0, "gnf_linear_wgrad_tc")
-    elif passes:
+    if passes:
         _note_flops("gnf_linear_wgrad_tc", 2. * M * N * K, (M, N, K))
         _call("gnf_linear_wgrad_tc", ptr(dY), lddy, ptr(X), ldx, ptr(dW), lddw, M, N, K, passes, stream_ptr())
     else:
@@ -550,7 +514,7 @@ def linear_wgrad(dY, lddy, X, ldx, M, N, K, dy_split=None, x_split=None, out=Non
 
 def linear_wgrad_bias(dY, lddy, X, ldx, M, N, K):
     """(dW, db) of one Linear layer; in 3xTF32 the weight-gradient engine takes db from the dY tiles it streams (one launch)."""
-    if _gemm_passes(M, N, K, "wgrad") == 3 and M > 0 and not PRESPLIT_ACTS:
+    if _gemm_passes(M, N, K, "wgrad") == 3 and M > 0:
         dW = torch.empty(N, K, device=dY.device, dtype=dY.dtype)
         db = torch.empty(N, device=dY.device, dtype=dY.dtype)
         _note_flops("gnf_linear_wgrad_tc", 2. * M * N * K, (M, N, K))
@@ -569,7 +533,7 @@ def colsum(Y, ldy, M, N, period=1):
     return out
 
 
-def _mlp_backward(gout, ldg, acts, x_in, ldx, K0, weights, need_dx, first_layer_done=False, act_splits=None):
+def _mlp_backward(gout, ldg, acts, x_in, ldx, K0, weights, need_dx, first_layer_done=False):
     """Shared backward of a Linear/ReLU stack.
 
     gout: cotangent of the last layer's (un-activated) output [M, N_last] with row stride ldg.
@@ -579,45 +543,30 @@ def _mlp_backward(gout, ldg, acts, x_in, ldx, K0, weights, need_dx, first_layer_
     M = gout.shape[0]
     dWs, dbs = [None] * n, [None] * n
     delta, ldd = gout, ldg
-    for l in range(n - 1, -1, -1):
+    for l in range(n - 1, 0, -1):
         W = weights[l]
         N, K = W.shape
-        if l == 0 and first_layer_done:
-            break
-        if l > 0 and not PRESPLIT_ACTS:
-            a_prev = acts[l - 1]
-            if _gemm_passes(M, N, K, "wgrad") == 0 and M > 0:
-                # a skinny layer on the FFMA engine (cfg4's 630 -> 30 output layer: ~20 us each, a fraction of the SMs): the weight / bias
-                # gradient and the input cotangent run side by side
-                with _Fork(0, delta) as f:
-                    dWs[l], dbs[l] = linear_wgrad_bias(delta, ldd, a_prev, a_prev.stride(0), M, N, K)
-                delta_in, delta = delta, linear_dgrad(delta, ldd, W, a_prev, M)
-                f.join()
-                del delta_in
-            else:
+        a_prev = acts[l - 1]
+        if _gemm_passes(M, N, K, "wgrad") == 0 and M > 0:
+            # a skinny layer on the FFMA engine (cfg4's 630 -> 30 output layer: ~20 us each, a fraction of the SMs): the weight / bias
+            # gradient and the input cotangent run side by side
+            with _Fork(0, delta) as f:
                 dWs[l], dbs[l] = linear_wgrad_bias(delta, ldd, a_prev, a_prev.stride(0), M, N, K)
-                delta = linear_dgrad(delta, ldd, W, a_prev, M)
-            ldd = delta.stride(0)
-            continue
-        dbs[l] = colsum(delta, ldd, M, N).view(N)
-        if l > 0:
-            a_prev = acts[l - 1]
-            # the cotangent is read by this layer's wgrad and dgrad: split it once for both (when they run pre-split at all)
-            xs = act_splits[l] if act_splits is not None else None
-            ds = None
-            if (PRESPLIT_ACTS and PRESPLIT_WEIGHTS and M > 0 and min(N, K) >= PRESPLIT_ACTS_MIN_K and _gemm_passes(M, N, K) == 3
-                    and _gemm_passes(M, N, K, "wgrad") == 3):
-                ds = _split_mat(delta, M, N, ldd)
-                if xs is None:
-                    xs = _split_mat(a_prev, M, K, a_prev.stride(0))
-            dWs[l] = linear_wgrad(delta, ldd, a_prev, a_prev.stride(0), M, N, K, dy_split=ds, x_split=xs if ds is not None else None)
-            delta = linear_dgrad(delta, ldd, W, a_prev, M, dy_split=ds)
-            ldd = delta.stride(0)
+            delta_in, delta = delta, linear_dgrad(delta, ldd, W, a_prev, M)
+            f.join()
+            del delta_in
         else:
-            dWs[0] = linear_wgrad(delta, ldd, x_in, ldx, M, N, K0)
-            dx = linear_dgrad(delta, ldd, W, None, M) if need_dx else None
-            return dWs, dbs, dx, delta
-    return dWs, dbs, None, delta
+            dWs[l], dbs[l] = linear_wgrad_bias(delta, ldd, a_prev, a_prev.stride(0), M, N, K)
+            delta = linear_dgrad(delta, ldd, W, a_prev, M)
+        ldd = delta.stride(0)
+    if first_layer_done:
+        return dWs, dbs, None, delta
+    W = weights[0]
+    N = W.shape[0]
+    dbs[0] = colsum(delta, ldd, M, N).view(N)
+    dWs[0] = linear_wgrad(delta, ldd, x_in, ldx, M, N, K0)
+    dx = linear_dgrad(delta, ldd, W, None, M) if need_dx else None
+    return dWs, dbs, dx, delta
 
 
 class MlpFn(torch.autograd.Function):
@@ -779,12 +728,10 @@ DAG_L1_NARROW_TC = True
 DAG_L1_NARROW_TC_FWD = True
 
 
-def _dag_l1_plane(M, N1, d, direction):
-    """direction 'fwd' / 'bwd'; DAG_L1_PLANE may also be the string 'fwd' or 'bwd' (measurement: one direction only)."""
-    on = DAG_L1_PLANE is True or DAG_L1_PLANE == direction
+def _dag_l1_plane(M, N1, d):
     # narrow flows (d <= 64) stay on the resident-gate kernels: through the plane + the register-tiled GEMM layer 1 of cfg4 measured
     # 43 / 45 / 73 us (forward / wgrad / dgrad) against 45 / 51 / 55 us, plus the plane kernels (profiles/r02aa_*)
-    return on and d >= DAG_L1_PLANE_MIN_D and M > 0 and _gemm_passes(M, N1, d) != 0 and not L._SIMULATOR
+    return DAG_L1_PLANE and d >= DAG_L1_PLANE_MIN_D and M > 0 and _gemm_passes(M, N1, d) != 0 and not L._SIMULATOR
 
 
 class DagMlpFn(torch.autograd.Function):
@@ -826,7 +773,7 @@ class DagMlpFn(torch.autograd.Function):
         g = gate.c_struct()
         # the weight splits of the hidden layers depend on nothing of this step: a side branch next to layer 1
         f_split = None
-        if PRESPLIT_WEIGHTS and not PRESPLIT_ACTS and B > 0:
+        if B > 0:
             todo = [weights[l] for l in range(1, n) if _gemm_passes(B * d, weights[l].shape[0], weights[l].shape[1]) == 3]
             if todo:
                 with _Fork(0, x) as f_split:
@@ -835,7 +782,7 @@ class DagMlpFn(torch.autograd.Function):
         y = _rows(B * d, N1, x) if n > 1 else torch.empty(B * d, N1, device=x.device, dtype=x.dtype)
         E = W1e = narrow = None
         gate_planes = (None, None)
-        if _dag_l1_plane(B * d, N1, d, "fwd"):
+        if _dag_l1_plane(B * d, N1, d):
             E = _rows(B * d, d, x)
             if DAG_L1_PLANE_KEEP_DERIVATIVES and (ctx.needs_input_grad[0] or ctx.needs_input_grad[1]):
                 gate_planes = (_rows(B * d, d, x), _rows(B * d, d, x))        # de/dx, de/dP (same row stride as E): the backward reduction streams them
@@ -866,15 +813,13 @@ class DagMlpFn(torch.autograd.Function):
         if f_split is not None:
             f_split.join()
         acts = []
-        splits = [None] * n       # splits[l] = TF32 (hi, lo) of layer l's input, when its forward GEMM ran pre-split: reused by its wgrad
         cur = y
         for l in range(1, n):
             acts.append(cur)
             out = None
             if l == n - 1:   # final layer writes straight into the [B, d, H] result (no view of an internal tensor)
                 out = torch.empty(B, d, weights[l].shape[0], device=x.device, dtype=x.dtype)
-            cur, splits[l] = linear_fwd(cur, weights[l], biases[l], relu=(l < n - 1), out=out, ldy=weights[l].shape[0], want_split=True)
-        ctx.act_splits = splits if any(ctx.needs_input_grad) else None
+            cur = linear_fwd(cur, weights[l], biases[l], relu=(l < n - 1), out=out, ldy=weights[l].shape[0])
         ctx.E, ctx.W1e = (E, W1e) if any(ctx.needs_input_grad) else (None, None)
         ctx.gate_planes = gate_planes
         ctx.narrow = narrow if any(ctx.needs_input_grad) else None
@@ -894,24 +839,15 @@ class DagMlpFn(torch.autograd.Function):
         B, d = x.shape
         M = B * d
         gh = _contig(gh).view(M, -1)
-        st = stream_ptr()
-        dWs, dbs, _, delta = _mlp_backward(gh, gh.stride(0), acts, None, 0, 0, weights, False, first_layer_done=True,
-                                           act_splits=ctx.act_splits)
-        ctx.act_splits = None
+        dWs, dbs, _, delta = _mlp_backward(gh, gh.stride(0), acts, None, 0, 0, weights, False, first_layer_done=True)
         W1 = weights[0]
         N1 = W1.shape[0]
         g = gate.c_struct()
         dW1 = torch.empty_like(W1)
-        E, W1e = ctx.E, ctx.W1e
+        E, W1e = ctx.E, ctx.W1e           # set iff the forward ran layer 1 against the embedding plane: the backward follows it
         DXp, DPp = ctx.gate_planes
         ctx.E = ctx.W1e = None
         ctx.gate_planes = (None, None)
-        if E is not None and not _dag_l1_plane(M, N1, d, "bwd"):
-            E = None
-        elif E is None and _dag_l1_plane(M, N1, d, "bwd"):        # forward ran on the loader kernels: regenerate the plane (same Philox counters)
-            E = _rows(M, d, x)
-            _call("gnf_dag_embed_fwd", ptr(x), ptr(P), C.byref(g), ptr(E), None, None, E.stride(0), B, d, st)
-            W1e = W1[:, :d]
         narrow, ctx.narrow = ctx.narrow, None
         narrow_tc = narrow is not None and _narrow_l1_tc(M, N1, delta)
         # three independent pieces: [weight gradient of the masked half] | [bias table -> one-hot half of dW1, db1] | [input cotangent]
@@ -1000,10 +936,9 @@ def _activation_budget(device):
 UMNN_ENGINE = "auto"
 UMNN_LAYERWISE_MIN_NODE_ROWS = 16384
 # The strict forward of the layer-wise engine runs as ONE fused tensor-core kernel (gnf_umnn_fwd_tc3) when the integrand fits it
-# (>= 3 linear layers, hidden widths <= 160); False = per-layer passes (gnf_umnn_fwd_lw).
+# (>= 3 linear layers, hidden widths <= 160); False = per-layer passes (gnf_umnn_fwd_lw).  Its backward runs the dgrad chain as one
+# fused tensor-core kernel too (gnf_umnn_bwd_tc3) whenever that kernel takes the shape, else gnf_umnn_bwd_lw.
 UMNN_FWD_FUSED_TC3 = True
-# ... and its backward runs the dgrad chain as one fused tensor-core kernel too (gnf_umnn_bwd_tc3); False = gnf_umnn_bwd_lw
-UMNN_BWD_FUSED_TC3 = True
 
 
 def _umnn_layerwise_passes(net, R, S, train, device=None):
@@ -1086,6 +1021,7 @@ class UmnnFn(torch.autograd.Function):
         zrev = torch.empty_like(x) if want_rev else None
         logdet = torch.empty(B, device=x.device, dtype=x.dtype)
         saved = None
+        fused_bwd = False
         train = any(ctx.needs_input_grad)
         lw_passes = None if fast else _umnn_layerwise_passes(net, R, int(S), train, x.device)
         if fast:
@@ -1099,7 +1035,7 @@ class UmnnFn(torch.autograd.Function):
             # cancelling sums amplify to 1e-3 .. 2e-3 on the integrand's bias gradients); evaluation = per-chunk order 0
             if train:
                 saved = torch.empty(lib().gnf_umnn_tc3_saved_floats(C.byref(net), R, int(S)), device=x.device, dtype=torch.float32)
-                ctx.fused_bwd = UMNN_BWD_FUSED_TC3 and lib().gnf_umnn_bwd_tc3_workspace_bytes(C.byref(net), R, int(S)) != 0
+                fused_bwd = lib().gnf_umnn_bwd_tc3_workspace_bytes(C.byref(net), R, int(S)) != 0
             nbytes = lib().gnf_umnn_tc3_workspace_bytes(C.byref(net), R)
             ws = torch.empty((nbytes + 3) // 4, device=x.device, dtype=torch.float32)
             _call("gnf_umnn_fwd_tc3", ptr(x), ptr(h), C.byref(net), int(S), ptr(ccw), ptr(ccn), ptr(z), ptr(zrev), ptr(jac),
@@ -1126,7 +1062,7 @@ class UmnnFn(torch.autograd.Function):
             _call("gnf_umnn_fwd", ptr(x), ptr(h), C.byref(net), int(S), ptr(ccw), ptr(ccn), ptr(z), ptr(zrev), ptr(jac),
                   ptr(logdet), ptr(saved), R, d, ptr(ws), nbytes, stream_ptr())
         ctx.lw_passes = lw_passes if (lw_passes is not None and train) else None
-        ctx.fused_bwd = getattr(ctx, "fused_bwd", False)
+        ctx.fused_bwd = fused_bwd
         _count(2)
         ctx.saved_acts = saved
         ctx.save_for_backward(x, h, jac, *weights, *biases)
@@ -1161,7 +1097,7 @@ class UmnnFn(torch.autograd.Function):
         for l in range(n):
             grads.dW[l] = dWs[l].data_ptr()
             grads.db[l] = dbs[l].data_ptr()
-        if ctx.lw_passes is not None and getattr(ctx, "fused_bwd", False):
+        if ctx.lw_passes is not None and ctx.fused_bwd:
             # dgrad chain fused on the tensor cores (tc_umnn3.cu), then the resident weight-gradient GEMMs
             nbytes = lib().gnf_umnn_bwd_tc3_workspace_bytes(C.byref(net), R, ctx.S)
             ws = torch.empty((nbytes + 3) // 4, device=x.device, dtype=torch.float32)

@@ -77,9 +77,6 @@ int gnf_nll_loss_fwd(const float* z, const float* logdet, const float* constrain
 /* gz[b,i] = z[b,i] g / B, glogdet[b] = -g / B (nullable); g: device scalar cotangent of the loss (NULL = 1). */
 int gnf_nll_loss_bwd(const float* z, const float* g, float* gz, float* glogdet, int B, int d, gnf_stream_t stream);
 
-/* log(jac).sum(1) for a jac [B,d] produced elsewhere (NormalizingFlow.py:70). */
-int gnf_logdet_fwd(const float* jac, float* logdet, int B, int d, gnf_stream_t stream);
-
 /* --------------------------------------------------------------------------------------------
  * K2 — acyclicity term  tr((I + alpha A∘A)^p) - d
  * (DAGConditioner.get_power_trace, models/Conditionners/DAGConditioner.py:176-194)
@@ -122,8 +119,6 @@ int gnf_linear_fwd_splitk(const float* X, int ldx, const float* W, int ldw, cons
                           int relu, void* work, size_t work_bytes, gnf_stream_t stream);
 /* out[p,n] = sum_{m % period == p} Y[m,n]  (bias gradients; one-hot column gradients). */
 int gnf_colsum(const float* Y, int ldy, float* out, int M, int N, int period, gnf_stream_t stream);
-/* dY[m,n] *= (act[m,n] > 0)  — ReLU backward for a cotangent produced outside the engine. */
-int gnf_relu_mask(float* dY, int lddy, const float* act, int ldact, int M, int N, gnf_stream_t stream);
 
 /* The same three GEMMs on the tensor cores (tcgen05.mma kind::tf32, fp32 accumulation in TMEM; warp-specialised
  * persistent kernel, operands staged into 128B-swizzled UMMA tiles by producer warps).
@@ -154,13 +149,6 @@ int gnf_linear_fwd_tc_ps_tb(const float* X, int ldx, const float* W_hi, const fl
                             int period, float* Y, int ldy, int M, int N, int K, int relu, gnf_stream_t stream);
 int gnf_linear_dgrad_tc_ps(const float* dY, int lddy, const float* W_hi, const float* W_lo, int ldw, const float* act, int ldact,
                            float* dX, int lddx, int M, int N, int K, gnf_stream_t stream);
-/* Both operands pre-split (gnf_split_tf32 on the activations as well: one 10-us elementwise pass per 16 MB operand, reused by the
- * GEMMs that consume it): nothing is split in shared memory, the MMA warp consumes the TMA tiles as they land.
- * op 0 = forward (A = X [M,K], B = W [N,K], bias / relu), 1 = dgrad (A = dY [M,N], B = W [N,K], act = ReLU mask source, C = dX),
- * 2 = wgrad (A = dY [M,N], B = X [M,K], C = dW [N,K]).  lda / ldb are the row strides of the hi AND lo arrays. */
-int gnf_linear_tc_ps2(int op, const float* A_hi, const float* A_lo, int lda, const float* B_hi, const float* B_lo, int ldb,
-                      const float* bias, int bias_period, const float* act, int ldact, float* C, int ldc, int M, int N, int K,
-                      int relu, gnf_stream_t stream);
 /* Host-only query of that plan for a GEMM of M x N outputs reduced over K (wgrad != 0: the split-K orientation, where M x N is
  * the weight shape and K the number of rows): writes the tile width and the split-K factor the engine would use. */
 int gnf_tc_gemm_plan(int M, int N, int K, int passes, int wgrad, int* bn, int* splits);
@@ -436,8 +424,6 @@ int gnf_reverse_cols(const float* src, float* dst, int B, int d, gnf_stream_t st
 int gnf_broadcast_rows(const float* constants, float* h, int B, int d, int indep, int H, gnf_stream_t stream);
 /* *counter += inc  (device-side Philox offset for graph-captured training steps). */
 int gnf_counter_add(uint64_t* counter, uint64_t inc, gnf_stream_t stream);
-/* y[i] += a * x[i]  (flat gradient bucket packing / scaling for the data-parallel all-reduce). */
-int gnf_axpy(float a, const float* x, float* y, size_t n, gnf_stream_t stream);
 
 #ifdef __cplusplus
 }

@@ -53,7 +53,8 @@ int gnf_tc_probe(int mode, int iters, long long* out, gnf_stream_t stream);
 /* Debug / measurement: later gnf_umnn_fwd_tc calls write per-phase SM-clock stamps of CTA 0 into buf (48*8 int64). */
 int gnf_tc_set_trace(long long* buf);
 
-/* 0 keeps the pre-split forward / dgrad GEMMs on the first engine (stagers split the activation tile in shared memory). */
+/* Measurement switch: 0 keeps the pre-split forward / dgrad GEMMs on the first engine (stagers split the activation tile in shared
+ * memory); 1 (default) = engine v2.  Any other value is GNF_ERR_INVALID. */
 int gnf_tc_gemm_set_v2(int enable);
 /* Fused strict UMNN forward (tc_umnn3.cu): CTA 0 records SM-clock stamps into buf[4][256] (rows: issuer, epilogue warp 0,
  * producer, epilogue warp of the last column block); NULL disables. */

@@ -32,8 +32,7 @@ def main(B=16, cfg="cfg5"):
         import devlib
         devlib.install().gnf_tc_gemm_set_fold(int(fold))
         print(f"fold = {fold}")
-    for name, gemm, plane in (("plane+tc", "auto", True), ("plane-fwd", "auto", "fwd"), ("plane-bwd", "auto", "bwd"), ("ffma-l1+tc", "auto", False),
-                              ("all-ffma", "ffma", True)):
+    for name, gemm, plane in (("plane+tc", "auto", True), ("ffma-l1+tc", "auto", False), ("all-ffma", "ffma", True)):
         G.ops.set_gemm_mode(gemm)
         G.ops.DAG_L1_PLANE = plane
         model = G.build_from_spec(spec, "cuda", 0)

@@ -34,7 +34,7 @@ def timed(fn, n=30):
     return e0.elapsed_time(e1) / n * 1000
 
 
-for v2 in (1, 2, 0):
+for v2 in (1, 0):
     lib.gnf_tc_gemm_set_v2(v2)
     for fold in (1, 2, 4, 1000):
         lib.gnf_tc_gemm_set_fold(fold)
@@ -44,7 +44,7 @@ for v2 in (1, 2, 0):
         err = float((Y.double() - ref).norm() / ref.norm())
         bias = float((Y.double() - ref).mean() / ref.abs().mean())
         worst = float((Y.double() - ref).abs().max() / ref.abs().mean())
-        print(f"engine v{('1', '2 (2 partials, 4 A buffers)', '2 (3 partials, 2 A buffers)')[v2]} fold={fold:4d}: fwd {f:6.1f} us  dgrad {d:6.1f} us   fwd rel L2 err {err:.2e}  mean signed err / mean |y| {bias:+.2e}"
+        print(f"engine v{('1', '2')[v2]} fold={fold:4d}: fwd {f:6.1f} us  dgrad {d:6.1f} us   fwd rel L2 err {err:.2e}  mean signed err / mean |y| {bias:+.2e}"
               f"  max |err| / mean |y| {worst:.2e}")
 lib.gnf_tc_gemm_set_fold(2)
 lib.gnf_tc_gemm_set_v2(1)

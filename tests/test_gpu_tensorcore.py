@@ -387,15 +387,3 @@ def test_rw_wgrad_exact_and_fp32_equivalent(M_, N, K):
         dW2 = G.ops.linear_wgrad_rw(_padded(dY, NPn), Xp, N, K, passes=3)
         assert torch.equal(dW2, dW)
 
-
-def test_fully_presplit_conditioner_gemms_vs_oracle(gemm_mode):
-    """gnf_linear_tc_ps2: both GEMM operands split into TF32 hi / lo in global memory (off by default, see ops.PRESPLIT_ACTS)."""
-    import model_vs_oracle as M
-    gemm_mode("tf32x3")
-    G.ops.PRESPLIT_ACTS = True
-    try:
-        rep = M.compare(M.CONFIGS["cfg4"], 24, "cuda", train=True)
-    finally:
-        G.ops.PRESPLIT_ACTS = False
-    bad = {k: v for k, v in rep.items() if (k.startswith("grad.") and not v < 1e-3) or (k in ("ll", "loss") and not v < 1e-4)}
-    assert not bad, bad
