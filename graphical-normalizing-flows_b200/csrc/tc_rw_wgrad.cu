@@ -376,9 +376,13 @@ bool rw_wgrad_supported(int N, int K) {
 int launch_rw_wgrad(const float* dY, long long lddy, const float* X, long long ldx, float* dW, long long lddw, int Q, int N, int K, int passes,
                     float* partial, cudaStream_t s, const Branches* br, int side, const RwRankOne* rank_one) {
   if (passes != 1 && passes != 3) return fail(GNF_ERR_INVALID, "resident wgrad: passes must be 1 or 3");
-  const int NP = (K + 31) / 32 * 32;
-  if (!rw_wgrad_supported(N, K) || ldx != NP || lddy < N || (reinterpret_cast<uintptr_t>(X) & 15) || (reinterpret_cast<uintptr_t>(partial) & 15))
-    return fail(GNF_ERR_UNSUPPORTED, "resident wgrad: needs N <= 160, K <= 160 and a dense 16-byte aligned activation plane (ld = %d)", NP);
+  // The kernel multiplies all ldx columns of X: the activation planes of a mixed-width integrand share the row stride of its widest
+  // layer, so a narrower layer's plane carries columns past round_up(K, 32); the reduction keeps the first K.  `partial` holds
+  // rw_wgrad_partial_floats(ldx) floats.
+  const int NP = (int)ldx;
+  if (K < 1 || ldx % 32 != 0 || ldx < (K + 31) / 32 * 32 || !rw_wgrad_supported(N, NP) || lddy < N || (reinterpret_cast<uintptr_t>(X) & 15) ||
+      (reinterpret_cast<uintptr_t>(partial) & 15))
+    return fail(GNF_ERR_UNSUPPORTED, "resident wgrad: needs N <= 160, K <= 160 and a dense 16-byte aligned activation plane (ld = %lld, K = %d)", ldx, K);
   if (Q <= 0) { cudaMemset2DAsync(dW, (size_t)lddw * sizeof(float), 0, (size_t)K * sizeof(float), (size_t)N, s); return 0; }
   const int nchunks = (Q + kWgQC - 1) / kWgQC;
   const int cpc = (nchunks + kNumSMs - 1) / kNumSMs;
@@ -438,6 +442,7 @@ int gnf_linear_wgrad_rw(const float* dY, int lddy, const float* X, int ldx, floa
 #else
   if (!dY || !X || !dW || M < 0 || N <= 0 || K <= 0 || lddw < K) return fail(GNF_ERR_INVALID, "gnf_linear_wgrad_rw: bad arguments");
   if (!rw_wgrad_supported(N, K)) return fail(GNF_ERR_UNSUPPORTED, "gnf_linear_wgrad_rw: %d x %d is out of range (N, K <= 160)", N, K);
+  if (ldx != (K + 31) / 32 * 32) return fail(GNF_ERR_UNSUPPORTED, "gnf_linear_wgrad_rw: X must be a dense plane (ldx = %d)", (K + 31) / 32 * 32);
   if (!work || work_bytes < rw_wgrad_partial_floats(K) * sizeof(float)) return fail(GNF_ERR_WORKSPACE, "gnf_linear_wgrad_rw: workspace too small");
   if (int e = launch_rw_wgrad(dY, lddy, X, ldx, dW, lddw, M, N, K, passes, (float*)work, (cudaStream_t)stream)) return e;
   return check_launch("gnf_linear_wgrad_rw");

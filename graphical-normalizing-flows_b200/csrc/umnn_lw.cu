@@ -658,7 +658,7 @@ int gnf_umnn_bwd_tc3(const float* x, const float* h, const gnf_mlp_t* net, int S
   zl.add(dx, (size_t)R);
   const Branches& br = branches();
   cudaStream_t pack_stream = br.ok ? br.begin(s, 0) : nullptr;     // the chain's weight images: next to the zero-fill and the output pass
-  zero_many(zl, s);                    // every gradient tensor, D and dx: one launch (GNF_MAX_LAYERS = 6: at most 14 entries)
+  zero_many(zl, s);                    // every gradient tensor, D and dx: one launch (GNF_MAX_LAYERS = 8: at most 18 entries)
   // output layer: g_q per node-row (the weight-gradient kernel of W_{L-1} rebuilds delta_L from it and the saved ReLU mask of a_L: no
   // delta_L plane), dW_L, db_L, db_{L-1}.  g_q lives in the first Q floats of what used to be that plane.
   float* gq = dplanes;

@@ -939,6 +939,13 @@ UMNN_LAYERWISE_MIN_NODE_ROWS = 16384
 # (>= 3 linear layers, hidden widths <= 160); False = per-layer passes (gnf_umnn_fwd_lw).  Its backward runs the dgrad chain as one
 # fused tensor-core kernel too (gnf_umnn_bwd_tc3) whenever that kernel takes the shape, else gnf_umnn_bwd_lw.
 UMNN_FWD_FUSED_TC3 = True
+# gnf_umnn_fwd_tc3 / gnf_umnn_bwd_tc3 stage the S + 1 quadrature nodes and weights in shared memory (kU3MaxNodes, tc_umnn3.cu)
+UMNN_TC3_MAX_NODES = 256
+
+
+def _umnn_tc3_takes(net, R, S):
+    """Does the fused strict forward (gnf_umnn_fwd_tc3) take this integrand at R rows and S quadrature steps?"""
+    return UMNN_FWD_FUSED_TC3 and S + 1 <= UMNN_TC3_MAX_NODES and lib().gnf_umnn_tc3_workspace_bytes(C.byref(net), R) != 0
 
 
 def _umnn_layerwise_passes(net, R, S, train, device=None):
@@ -1027,7 +1034,7 @@ class UmnnFn(torch.autograd.Function):
         if fast:
             _call("gnf_umnn_fwd_tc", ptr(x), ptr(h), C.byref(net), int(S), ptr(ccw), ptr(ccn), ptr(z), ptr(zrev), ptr(jac),
                   ptr(logdet), R, d, ptr(ws), nbytes, stream_ptr())
-        elif lw_passes == 3 and UMNN_FWD_FUSED_TC3 and lib().gnf_umnn_tc3_workspace_bytes(C.byref(net), R) != 0:
+        elif lw_passes == 3 and _umnn_tc3_takes(net, R, int(S)):
             # fused strict forward (tc_umnn3.cu): 3xTF32, the activation chain of a tile stays in TMEM from the first to the
             # last hidden layer; training keeps the planes / masks the layer-wise backward consumes, evaluation keeps nothing.
             # MMA order: training = all correction products of a layer first (order 1: 20 instead of 60 truncating additions at
@@ -1128,8 +1135,7 @@ def umnn_forward_on_tensor_cores(params, R, S, device):
         return False
     weights, biases = [p.detach() for p in params[0::2]], [p.detach() for p in params[1::2]]
     net = _mlp_struct(weights, biases)
-    return (_umnn_layerwise_passes(net, R, int(S), False, device) == 3 and UMNN_FWD_FUSED_TC3
-            and lib().gnf_umnn_tc3_workspace_bytes(C.byref(net), R) != 0)
+    return _umnn_layerwise_passes(net, R, int(S), False, device) == 3 and _umnn_tc3_takes(net, R, int(S))
 
 
 def umnn_invert(z, h, S, weights, biases, iters=20, lo=-20., hi=20.):

@@ -280,7 +280,7 @@ int gnf_umnn_fwd(const float* x, const float* h, const gnf_mlp_t* net, int S, co
  * every quadrature node of its rows: needs S + 1 <= 64); lo / hi = the initial interval, x = midpoint of the final one. */
 int gnf_umnn_invert(const float* z, const float* h, const gnf_mlp_t* net, int S, const float* ccw, const float* ccn, float* x,
                     int iters, float lo, float hi, int R, void* work, size_t work_bytes, gnf_stream_t stream);
-/* Cotangents: gz [R], gzrev [R] (nullable), gjac [R] (nullable), glogdet [R/d] (nullable).
+/* Cotangents: gz [R], gzrev [R], gjac [R], glogdet [R/d], each nullable (NULL = zero cotangent).
  * Gradient convention = UMNN's: dtheta, dh by quadrature of the integrand's gradients with weights
  * w_k*gz*x/2; dx by the Leibniz rule f(x)*gz; the jac output is differentiated by the plain chain rule. */
 int gnf_umnn_bwd(const float* x, const float* h, const gnf_mlp_t* net, int S, const float* ccw, const float* ccn,
