@@ -894,7 +894,8 @@ __global__ void __launch_bounds__(kG2Threads, 1) tc_gemm2_kernel(TcGemmParams p,
 #pragma unroll
               for (int e = 0; e < 32; ++e) {
                 const int nb = n0 + c + e;
-                bv[e] = __ldg(p.bias + (nb < p.N ? nb : p.N - 1));       // columns >= N are never stored
+                const float b = __ldg(p.bias + (nb < p.N ? nb : p.N - 1));
+                bv[e] = nb < p.N ? b : 0.f;           // columns >= N of a piece straddling N are stored: they must stay 0
               }
             } else {
 #pragma unroll
@@ -929,13 +930,16 @@ __global__ void __launch_bounds__(kG2Threads, 1) tc_gemm2_kernel(TcGemmParams p,
           for (int i = 0; i < 8; ++i) {
             const int R = 4 * i + sub, m = m0 + R;
             uint4 o = *reinterpret_cast<const uint4*>(stage + R * 32 + 4 * (piece ^ (R & 7)));
-            if (m < p.M && n < p.N) {                    // pieces straddling N end in the row's padding (ldc >= round_up(N, 4)): zeros
+            // pieces straddling N end in the row's padding (ldc >= round_up(N, 4)): their columns >= N get zeros (the accumulator is
+            // zero there -- B's rows >= N are TMA zero fill -- and so are the bias values selected for them)
+            if (m < p.M && n < p.N) {
               if (mask) {
                 const uint32_t mb = mbits[c >> 5] >> (4 * i);
                 o.x = (mb & 1u) ? o.x : 0u; o.y = (mb & 2u) ? o.y : 0u; o.z = (mb & 4u) ? o.z : 0u; o.w = (mb & 8u) ? o.w : 0u;
-              } else if (table) {                        // N % 4 == 0 here (g2_eligible): the piece is inside the table row
-                const float4 b4 = tb[i];
-                float v0 = __uint_as_float(o.x) + b4.x, v1 = __uint_as_float(o.y) + b4.y, v2 = __uint_as_float(o.z) + b4.z, v3 = __uint_as_float(o.w) + b4.w;
+              } else if (table) {                        // bias_ld >= round_up(N, 4) (g2_eligible): the piece is inside the padded table row,
+                const float4 b4 = tb[i];                 // whose padding columns hold anything
+                float v0 = __uint_as_float(o.x) + b4.x, v1 = __uint_as_float(o.y) + (n + 1 < p.N ? b4.y : 0.f),
+                      v2 = __uint_as_float(o.z) + (n + 2 < p.N ? b4.z : 0.f), v3 = __uint_as_float(o.w) + (n + 3 < p.N ? b4.w : 0.f);
                 if (p.relu) { v0 = fmaxf(v0, 0.f); v1 = fmaxf(v1, 0.f); v2 = fmaxf(v2, 0.f); v3 = fmaxf(v3, 0.f); }
                 o = make_uint4(__float_as_uint(v0), __float_as_uint(v1), __float_as_uint(v2), __float_as_uint(v3));
               }

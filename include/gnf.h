@@ -123,7 +123,10 @@ int gnf_colsum(const float* Y, int ldy, float* out, int M, int N, int period, gn
 /* The same three GEMMs on the tensor cores (tcgen05.mma kind::tf32, fp32 accumulation in TMEM; warp-specialised
  * persistent kernel, operands staged into 128B-swizzled UMMA tiles by producer warps).
  *   passes = 1: single-pass TF32 (fast mode, log-likelihood tolerance 2e-3);
- *   passes = 3: 3xTF32 hi/lo split, fp32-equivalent (strict mode: ll 1e-4, gradients 1e-3). */
+ *   passes = 3: 3xTF32 hi/lo split, fp32-equivalent (strict mode: ll 1e-4, gradients 1e-3).
+ * Forward and dgrad (here and in the _ps / _ps_tb flavours below) store rows in 16-byte pieces: when ldy / lddx leave room for
+ * them, they may write zeros into the output columns [N, round_up(N, 4)) (dgrad: [K, round_up(K, 4))), and never write past
+ * them.  The weight gradients write the first K columns of dW only. */
 int gnf_linear_fwd_tc(const float* X, int ldx, const float* W, int ldw, const float* bias, int bias_period, float* Y,
                       int ldy, int M, int N, int K, int relu, int passes, gnf_stream_t stream);
 int gnf_linear_dgrad_tc(const float* dY, int lddy, const float* W, int ldw, const float* act, int ldact, float* dX,
