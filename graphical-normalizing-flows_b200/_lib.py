@@ -119,11 +119,8 @@ _PROTOS = {
     "gnf_umnn_bwd_tc3": ([_P, _P, C.POINTER(MlpT), _I, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, C.POINTER(MlpGradT), _I, _I,
                           _P, _SZ, _P], C.c_int),
     "gnf_umnn_fwd_tc3": ([_P, _P, C.POINTER(MlpT), _I, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _P, _SZ, _P], C.c_int),
-    "gnf_linear_rw_workspace_bytes": ([_I, _I], _SZ),
     "gnf_linear_wgrad_rw_workspace_bytes": ([_I, _I], _SZ),
     "gnf_linear_wgrad_rw": ([_P, _I, _P, _I, _P, _I, _I, _I, _I, _I, _P, _SZ, _P], C.c_int),
-    "gnf_linear_fwd_rw": ([_P, _I, _P, _I, _P, _P, _I, _P, _I, _I, _I, _I, _I, _P, _SZ, _P], C.c_int),
-    "gnf_linear_dgrad_rw": ([_P, _I, _P, _I, _P, _I, _P, _P, _I, _I, _I, _I, _I, _P, _SZ, _P], C.c_int),
     "gnf_tc_gemm_plan": ([_I, _I, _I, _I, _I, _P, _P], C.c_int),
     "gnf_tc_selftest": ([_P, _P, _P, _I, _I, _I, _P], C.c_int),
     "gnf_reverse_cols": ([_P, _P, _I, _I, _P], C.c_int),

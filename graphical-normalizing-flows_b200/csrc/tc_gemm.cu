@@ -667,8 +667,8 @@ __global__ void split_tf32_kernel(const float* __restrict__ W, long long ldw, fl
 //     partial accumulators in TMEM, folded every `fold` k-chunks into a round-to-nearest running sum that EIGHT epilogue
 //     warps (two per lane quarter, 64 columns each) keep in registers, so that a fold is one TMEM read + 64 additions and the
 //     output pass of a tile hides behind the next tile's first groups; correction products go first inside every chunk;
-//   * the final epilogue moves 32-column blocks through a 4 KB XOR-swizzled staging block per warp (rw_gemm_kernel's):
-//     every global instruction covers 4 rows x 128 bytes, the dgrad ReLU mask is applied on the coalesced side.
+//   * the final epilogue moves 32-column blocks through a 4 KB XOR-swizzled staging block per warp (DESIGN §4, row-owner
+//     note): every global instruction covers 4 rows x 128 bytes, the dgrad ReLU mask is applied on the coalesced side.
 // TMEM columns: partials 0 / 128, A ring 256 (four buffers of hi 32 + lo 32).
 // =====================================================================================================================
 constexpr int kG2BN = 128, kG2Stages = 4, kG2Threads = 14 * 32;   // 8 epilogue + 4 A-writer + MMA issuer + TMA producer warps

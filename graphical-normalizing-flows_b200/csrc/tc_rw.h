@@ -1,35 +1,11 @@
-// Internal interface of the resident-weight tcgen05 layer GEMM (tc_rw.cu) for the other translation units.
+// Internal interface of the resident weight-gradient tcgen05 kernel (tc_rw_wgrad.cu) for the other translation units.
 #pragma once
 #include "common.cuh"
 
 #ifndef GNF_EMU
 namespace gnf {
 
-enum { RW_EPI_BIAS_ACT = 0, RW_EPI_MASK = 1 };
-
-struct RwGemmParams {
-  // C[m, 0:NP) = epi( sum_{k < KP} A[m, k] * B[n, k] ),  B given as the packed image of rw_pack_image()
-  const float* A; long long lda;        // [M][lda] row-major, 16-byte aligned rows, KP columns readable (pad columns = 0)
-  float* C; long long ldc;              // [M][ldc], NP columns written (pad columns receive epi(0))
-  const float* image;                   // rw_image_floats(NP, KP) floats: hi image, lo image, bias[NP]
-  int M, NP, KP, passes, epi, relu;
-  const uint32_t* mask_bits; long long mask_ld;   // RW_EPI_MASK: keep C where bit n of row m is set ([M][mask_ld] words) ...
-  const float* act; long long ldact;              // ... or where act[m, n] > 0 (used when mask_bits is NULL)
-  uint32_t* bits_out; long long bits_ld;          // RW_EPI_BIAS_ACT: also emit the bit mask (C > 0), same layout
-  int debug;                                      // measurement (gnf_linear_rw_set_debug): skip stores / loads / MMAs
-  long long* trace;                               // measurement (set by launch_rw_gemm from gnf_linear_rw_set_trace)
-};
-
-static inline size_t rw_image_floats(int NP, int KP) { return (size_t)2 * NP * KP + NP; }
-// Can the resident-weight kernel run an (N x K) layer?  NP/KP = widths padded to 32.
-bool rw_supported(int N, int K);
-// image <- hi/lo split of W (transpose = 0: B[n,k] = W[n*ldw + k], W is [N][K]; 1: B[n,k] = W[k*ldw + n], W is [K][N])
-// zero padded to NP x KP, + bias (nullable) padded to NP.
-void rw_pack_image(const float* W, long long ldw, int N, int K, int transpose, const float* bias, float* image, int NP, int KP,
-                   cudaStream_t s);
-int launch_rw_gemm(const RwGemmParams& p, cudaStream_t s);
-
-// tc_rw_wgrad.cu: dW[N x K] = dY^T X over Q rows (N, K <= 160; X a dense [Q][pad32(K)] plane), partial tiles in `partial`
+// dW[N x K] = dY^T X over Q rows (N, K <= 160; X a dense [Q][pad32(K)] plane), partial tiles in `partial`
 // (rw_wgrad_partial_floats(K) floats), summed by a second kernel.
 bool rw_wgrad_supported(int N, int K);
 size_t rw_wgrad_partial_floats(int K);

@@ -17,9 +17,9 @@
 //   * the epilogue drains the accumulator (tcgen05.ld), adds the bias, applies ReLU and rewrites the A region for the
 //     next layer; after the last hidden layer it takes the output Linear as a dot product, ELU + 1.05, the CC
 //     weighting and the per-row segment reduction, emitting z, jac, logdet (+ zrev).
-// Training keeps what the layer-wise backward (gnf_umnn_bwd_lw) consumes, in its layout: the activation planes, the
-// pre-ELU outputs and the ReLU bit masks, written with full 128-byte lines through a per-warp XOR-swizzled staging
-// block (row-owner global stores are poison: see tc_rw.cu).
+// Training keeps what the backward (gnf_umnn_bwd_tc3) consumes, in the layer-wise engine's layout: the activation planes,
+// the pre-ELU outputs and the ReLU bit masks, written with full 128-byte lines through a per-warp XOR-swizzled staging
+// block (row-owner global stores are poison: DESIGN §4, "What the measurements said").
 #include "tc_common.cuh"
 
 #ifndef GNF_EMU
@@ -484,7 +484,7 @@ __global__ void __launch_bounds__((4 * NB + 2) * 32, 1) umnn_fwd_tc3_kernel(U3Pa
 // What leaves the chip: the delta_l planes the weight-gradient GEMMs (tc_rw_wgrad.cu) consume (l >= 2), the column sums
 // db_{l-1} = sum_q delta_l, and the first-layer reductions D[r] = sum_k delta_1[(r,k)], dW0[:,0] = sum_q delta_1[q] t_q,
 // dx[r] = delta_1[(r,S+1)] . W0[:,0] + jac[r] gz[r] -- taken with warp shuffles (16 columns x 32 rows per pass) and atomics.
-// Replaces two resident-weight dgrad GEMMs, the colsum pass and the layer-1 reduction pass of gnf_umnn_bwd_lw.
+// Replaces the dgrad GEMMs, the colsum passes and the layer-1 reduction pass of gnf_umnn_bwd_lw.
 // =====================================================================================================================
 struct U3BParams {
   const float *x, *ccw, *ccn, *jac, *gz, *gzrev, *gjac, *glogdet, *image, *saved;

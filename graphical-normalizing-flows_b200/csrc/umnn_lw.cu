@@ -335,14 +335,10 @@ __global__ void lw_finish_dh_kernel(float* __restrict__ dh, int E, const float* 
   for (int r = blockIdx.x * blockDim.x + threadIdx.x; r < R; r += gridDim.x * blockDim.x) dh[(size_t)r * E] += lw_gz_total(gz, gzrev, r, d);
 }
 
-static int g_lw_use_rw_wgrad = 1;   // measurement switch (gnf_umnn_lw_set_rw bit 1): 0 = wgrad on the generic tensor-core engine
-static int g_lw_use_rw = 1;   // measurement switch (gnf_umnn_lw_set_rw): 0 = hidden GEMMs on the generic tensor-core engine
-
 struct LwPlan {
   int L, NP, E, nodes;
-  int rw;          // hidden layers fit the resident-weight tensor-core kernel (tc_rw.cu)
   long long Q;
-  size_t off_P, off_Wp[GNF_MAX_LAYERS], off_dA, off_dB, off_D, off_part, total;  // workspace offsets in floats
+  size_t off_P, off_Wp[GNF_MAX_LAYERS], off_dA, off_dB, off_D, total;  // workspace offsets in floats
 };
 
 static int lw_plan(const gnf_mlp_t* net, int R, int S, int train, int backward, LwPlan* pl) {
@@ -364,23 +360,11 @@ static int lw_plan(const gnf_mlp_t* net, int R, int S, int train, int backward, 
   const size_t plane = (size_t)pl->Q * pl->NP;
   pl->off_P = off; off += (size_t)R * pl->NP;            // forward: P;  backward: D (same shape)
   pl->off_D = pl->off_P;
-#ifdef GNF_EMU
-  pl->rw = 0;
-#else
-  pl->rw = 1;                                              // every hidden layer, both directions (dgrad swaps N and K)
-  for (int l = 1; l < L; ++l)
-    if (!rw_supported(net->dims[l + 1], net->dims[l]) || !rw_supported(net->dims[l], net->dims[l + 1])) pl->rw = 0;
-#endif
-  // per hidden layer: the zero-padded weight copy (generic engines) or the hi/lo TF32 images + bias (resident-weight kernel)
-  for (int l = 1; l < L; ++l) { pl->off_Wp[l] = off; off += (size_t)2 * pl->NP * pl->NP + pl->NP; }
+  for (int l = 1; l < L; ++l) { pl->off_Wp[l] = off; off += (size_t)pl->NP * pl->NP; }   // zero-padded copy of each hidden weight
   pl->off_dA = pl->off_dB = 0;
-  pl->off_part = 0;
   if (backward) {
     pl->off_dA = off; off += plane;
     pl->off_dB = off; off += plane;
-#ifndef GNF_EMU
-    if (pl->rw) { pl->off_part = off; off += rw_wgrad_partial_floats(pl->NP); }   // per-CTA partial tiles of the wgrad kernel
-#endif
   }
   pl->total = off;
   return 0;
@@ -396,19 +380,11 @@ static inline int lw_blocks(long long work_items, int per_block, int max_per_sm)
 // Y = act(X W^T + b) / dX = (dY W) o relu'(act) / dW = dY^T X through the selected GEMM engine.
 // passes: 0 = strict FFMA tile GEMM, 1 = TF32, 3 = 3xTF32 (tcgen05).
 static int lw_fwd_gemm(const float* X, int ldx, const float* W, int ldw, const float* bias, float* Y, int ldy, int M, int N, int K,
-                       int relu, uint32_t* bits_out, int bits_ld, int passes, int rw_np, cudaStream_t s) {
+                       int relu, uint32_t* bits_out, int bits_ld, int passes, cudaStream_t s) {
   if (passes == 0) return gnf_linear_fwd(X, ldx, W, ldw, bias, 1, Y, ldy, M, N, K, relu, (gnf_stream_t)s);
 #ifdef GNF_EMU
   return fail(GNF_ERR_UNSUPPORTED, "tensor-core kernels have no host-simulator flavour");
 #else
-  if (rw_np) {                                           // W = packed hi/lo images + bias (rw_pack_image)
-    RwGemmParams r = {};
-    r.A = X; r.lda = ldx; r.C = Y; r.ldc = ldy; r.image = W;
-    r.M = M; r.NP = rw_np; r.KP = (K + 7) / 8 * 8; r.passes = passes; r.epi = RW_EPI_BIAS_ACT; r.relu = relu;
-    r.bits_out = bits_out; r.bits_ld = bits_ld;
-    if (int e = launch_rw_gemm(r, s)) return e;
-    return check_launch("gnf_umnn_fwd_lw (resident-weight GEMM)");
-  }
   TcGemmParams p = {};
   p.A = X; p.lda = ldx; p.a_src = TCG_SRC_K;
   p.B = W; p.ldb = ldw; p.b_src = TCG_SRC_K;
@@ -420,19 +396,11 @@ static int lw_fwd_gemm(const float* X, int ldx, const float* W, int ldw, const f
 #endif
 }
 static int lw_dgrad_gemm(const float* dY, int lddy, const float* W, int ldw, const float* act, int ldact, const uint32_t* mask_bits,
-                         int mask_ld, float* dX, int lddx, int M, int N, int K, int passes, int rw_np, cudaStream_t s) {
+                         int mask_ld, float* dX, int lddx, int M, int N, int K, int passes, cudaStream_t s) {
   if (passes == 0) return gnf_linear_dgrad(dY, lddy, W, ldw, act, ldact, dX, lddx, M, N, K, (gnf_stream_t)s);
 #ifdef GNF_EMU
   return fail(GNF_ERR_UNSUPPORTED, "tensor-core kernels have no host-simulator flavour");
 #else
-  if (rw_np) {                                           // W = packed hi/lo images of the TRANSPOSED weights
-    RwGemmParams r = {};
-    r.A = dY; r.lda = lddy; r.C = dX; r.ldc = lddx; r.image = W;
-    r.M = M; r.NP = rw_np; r.KP = (N + 7) / 8 * 8; r.passes = passes; r.epi = RW_EPI_MASK;   // reduction over the out-features
-    r.mask_bits = mask_bits; r.mask_ld = mask_ld; r.act = act; r.ldact = ldact;
-    if (int e = launch_rw_gemm(r, s)) return e;
-    return check_launch("gnf_umnn_bwd_lw (resident-weight GEMM)");
-  }
   TcGemmParams p = {};
   p.A = dY; p.lda = lddy; p.a_src = TCG_SRC_K;
   p.B = W; p.ldb = ldw; p.b_src = TCG_SRC_MN;
@@ -443,28 +411,14 @@ static int lw_dgrad_gemm(const float* dY, int lddy, const float* W, int ldw, con
 #endif
 }
 static int lw_wgrad_gemm(const float* dY, int lddy, const float* X, int ldx, float* dW, int lddw, int M, int N, int K, int passes,
-                         float* rw_partial, cudaStream_t s) {
+                         cudaStream_t s) {
   if (passes == 0) return gnf_linear_wgrad(dY, lddy, X, ldx, dW, lddw, M, N, K, (gnf_stream_t)s);
-#ifndef GNF_EMU
-  if (rw_partial) {                                      // lane = output row: dY^T goes to TMEM untransposed (tc_rw_wgrad.cu)
-    if (int e = launch_rw_wgrad(dY, lddy, X, ldx, dW, lddw, M, N, K, passes, rw_partial, s)) return e;
-    return check_launch("gnf_umnn_bwd_lw (resident wgrad)");
-  }
-#endif
   return gnf_linear_wgrad_tc(dY, lddy, X, ldx, dW, lddw, M, N, K, passes, (gnf_stream_t)s);
 }
 
-// Per-call weight staging of the hidden layers: hi/lo TF32 images for the resident-weight kernel (transposed for the
-// dgrad direction), else zero-padded copies for the generic engines.
-static void lw_pad_weights(const gnf_mlp_t* net, const LwPlan& pl, float* ws, int use_rw, int transpose, cudaStream_t s) {
+// Per-call weight staging of the hidden layers: zero-padded copies, read by both GEMM orientations.
+static void lw_pad_weights(const gnf_mlp_t* net, const LwPlan& pl, float* ws, cudaStream_t s) {
   for (int l = 1; l < pl.L; ++l) {
-#ifndef GNF_EMU
-    if (use_rw) {
-      if (transpose) rw_pack_image(net->W[l], net->dims[l], net->dims[l], net->dims[l + 1], 1, nullptr, ws + pl.off_Wp[l], pl.NP, (net->dims[l + 1] + 7) / 8 * 8, s);
-      else rw_pack_image(net->W[l], net->dims[l], net->dims[l + 1], net->dims[l], 0, net->b[l], ws + pl.off_Wp[l], pl.NP, (net->dims[l] + 7) / 8 * 8, s);
-      continue;
-    }
-#endif
     GNF_LAUNCH(lw_pad_weight_kernel, lw_blocks((long long)pl.NP * pl.NP, 256, 2), 256, 0, s, net->W[l], net->dims[l + 1], net->dims[l],
                ws + pl.off_Wp[l], pl.NP, pl.NP);
   }
@@ -475,14 +429,6 @@ static void lw_pad_weights(const gnf_mlp_t* net, const LwPlan& pl, float* ws, in
 using namespace gnf;
 
 extern "C" {
-
-#ifdef GNF_DEVTOOLS
-int gnf_umnn_lw_set_rw(int enable) {
-  g_lw_use_rw = (enable & 1) != 0;
-  g_lw_use_rw_wgrad = (enable & 1) != 0 && (enable & 2) == 0;      // 1: everything resident; 3: forward/dgrad only; 0: generic engine
-  return 0;
-}
-#endif
 
 size_t gnf_umnn_lw_saved_floats(const gnf_mlp_t* net, int R, int S, int train) {
   LwPlan pl;
@@ -516,8 +462,7 @@ int gnf_umnn_fwd_lw(const float* x, const float* h, const gnf_mlp_t* net, int S,
   // P = h W0[:,1:]^T + b0  (once per row r; strict fp32 on the FFMA engine: R x N1 x E is tiny)
   float* P = ws + pl.off_P;
   if (int e = gnf_linear_fwd(h, E, net->W[0] + 1, 1 + E, net->b[0], 1, P, NP, R, net->dims[1], E, 0, stream)) return e;
-  const int use_rw = (pl.rw && passes != 0 && g_lw_use_rw) ? 1 : 0;
-  lw_pad_weights(net, pl, ws, use_rw, 0, s);
+  lw_pad_weights(net, pl, ws, s);
   // ReLU bit masks of a_1 .. a_{L-1} (what the backward's dgrad epilogues consume), kept only when training on the tensor cores
   const int WB = NP / 32;
   const size_t bplane = (size_t)pl.Q * WB;
@@ -527,7 +472,7 @@ int gnf_umnn_fwd_lw(const float* x, const float* h, const gnf_mlp_t* net, int S,
   for (int l = 1; l < L; ++l) {
     uint32_t* bo = (bits && l + 1 < L) ? bits + (size_t)l * bplane : nullptr;     // mask of a_{l+1}
     if (int e = lw_fwd_gemm(saved + (size_t)(l - 1) * plane, NP, ws + pl.off_Wp[l], NP, net->b[l], saved + (size_t)l * plane, NP,
-                            (int)pl.Q, net->dims[l + 1], net->dims[l], 1, bo, WB, passes, use_rw ? NP : 0, s)) return e;
+                            (int)pl.Q, net->dims[l + 1], net->dims[l], 1, bo, WB, passes, s)) return e;
   }
   float* ysave = saved + (size_t)L * plane;
   {
@@ -561,8 +506,7 @@ int gnf_umnn_bwd_lw(const float* x, const float* h, const gnf_mlp_t* net, int S,
   const size_t plane = (size_t)pl.Q * NP;
   LwGeom g;
   g.R = R; g.d = d; g.E = E; g.S = S; g.nodes = pl.nodes; g.NP = NP; g.L = L; g.Q = pl.Q;
-  const int use_rw = (pl.rw && passes != 0 && g_lw_use_rw) ? 1 : 0;
-  lw_pad_weights(net, pl, ws, use_rw, 1, s);
+  lw_pad_weights(net, pl, ws, s);
   float* dcur = ws + pl.off_dA;
   float* dnxt = ws + pl.off_dB;
   const int red_threads = (NP / 4) * kLwRL;
@@ -577,10 +521,9 @@ int gnf_umnn_bwd_lw(const float* x, const float* h, const gnf_mlp_t* net, int S,
   // hidden layers, top down: dW_l = delta_{l+1}^T a_l;  delta_l = (delta_{l+1} W_l) o relu'(a_l);  db_{l-1} = colsum delta_l
   for (int l = L - 1; l >= 1; --l) {
     const float* a_l = saved + (size_t)(l - 1) * plane;
-    if (int e = lw_wgrad_gemm(dcur, NP, a_l, NP, grads->dW[l], net->dims[l], (int)pl.Q, net->dims[l + 1], net->dims[l], passes,
-                              (use_rw && g_lw_use_rw_wgrad) ? ws + pl.off_part : nullptr, s)) return e;
+    if (int e = lw_wgrad_gemm(dcur, NP, a_l, NP, grads->dW[l], net->dims[l], (int)pl.Q, net->dims[l + 1], net->dims[l], passes, s)) return e;
     const uint32_t* mb = passes != 0 ? reinterpret_cast<const uint32_t*>(saved + (size_t)L * plane + pl.Q) + (size_t)(l - 1) * pl.Q * (NP / 32) : nullptr;
-    if (int e = lw_dgrad_gemm(dcur, NP, ws + pl.off_Wp[l], NP, a_l, NP, mb, NP / 32, dnxt, NP, (int)pl.Q, net->dims[l + 1], net->dims[l], passes, use_rw ? NP : 0, s)) return e;
+    if (int e = lw_dgrad_gemm(dcur, NP, ws + pl.off_Wp[l], NP, a_l, NP, mb, NP / 32, dnxt, NP, (int)pl.Q, net->dims[l + 1], net->dims[l], passes, s)) return e;
     if (l > 1) {
       if (int e = gnf_colsum(dnxt, NP, grads->db[l - 1], (int)pl.Q, net->dims[l], 1, stream)) return e;
     }
@@ -614,7 +557,13 @@ size_t gnf_umnn_bwd_tc3_workspace_bytes(const gnf_mlp_t* net, int R, int S) {
   if (lw_plan(net, R, S, 1, 1, &pl)) return 0;
   const size_t img = u3_bwd_image_floats(net);
   if (img == 0) return 0;
-  if (!pl.rw) { set_error("umnn tc3 backward: the hidden layers do not fit the resident weight-gradient kernel"); return 0; }
+  // the weight gradient of every hidden GEMM layer runs on the resident wgrad kernel, over activation planes of row stride NP
+  for (int l = 1; l < pl.L; ++l)
+    if (!rw_wgrad_supported(net->dims[l + 1], pl.NP)) {
+      set_error("umnn tc3 backward: hidden layer %d (%d x %d, planes padded to %d) does not fit the resident weight-gradient kernel",
+                l, net->dims[l + 1], net->dims[l], pl.NP);
+      return 0;
+    }
   const size_t plane = (size_t)pl.Q * pl.NP;
   return ((size_t)R * pl.NP + (size_t)(pl.L - 1) * plane + 2 * (rw_wgrad_partial_floats(pl.NP) + 4) + img + 8) * sizeof(float);
 #endif

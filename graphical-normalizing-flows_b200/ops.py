@@ -1028,7 +1028,7 @@ class UmnnFn(torch.autograd.Function):
         zrev = torch.empty_like(x) if want_rev else None
         logdet = torch.empty(B, device=x.device, dtype=x.dtype)
         saved = None
-        fused_bwd = False
+        tc3 = False
         train = any(ctx.needs_input_grad)
         lw_passes = None if fast else _umnn_layerwise_passes(net, R, int(S), train, x.device)
         if fast:
@@ -1036,13 +1036,13 @@ class UmnnFn(torch.autograd.Function):
                   ptr(logdet), R, d, ptr(ws), nbytes, stream_ptr())
         elif lw_passes == 3 and _umnn_tc3_takes(net, R, int(S)):
             # fused strict forward (tc_umnn3.cu): 3xTF32, the activation chain of a tile stays in TMEM from the first to the
-            # last hidden layer; training keeps the planes / masks the layer-wise backward consumes, evaluation keeps nothing.
+            # last hidden layer; training keeps the planes / masks gnf_umnn_bwd_tc3 consumes, evaluation keeps nothing.
             # MMA order: training = all correction products of a layer first (order 1: 20 instead of 60 truncating additions at
             # full accumulator magnitude; with order 0 the saved activations carry a one-sided 5e-7 error that the backward's
             # cancelling sums amplify to 1e-3 .. 2e-3 on the integrand's bias gradients); evaluation = per-chunk order 0
+            tc3 = True
             if train:
                 saved = torch.empty(lib().gnf_umnn_tc3_saved_floats(C.byref(net), R, int(S)), device=x.device, dtype=torch.float32)
-                fused_bwd = lib().gnf_umnn_bwd_tc3_workspace_bytes(C.byref(net), R, int(S)) != 0
             nbytes = lib().gnf_umnn_tc3_workspace_bytes(C.byref(net), R)
             ws = torch.empty((nbytes + 3) // 4, device=x.device, dtype=torch.float32)
             _call("gnf_umnn_fwd_tc3", ptr(x), ptr(h), C.byref(net), int(S), ptr(ccw), ptr(ccn), ptr(z), ptr(zrev), ptr(jac),
@@ -1069,7 +1069,7 @@ class UmnnFn(torch.autograd.Function):
             _call("gnf_umnn_fwd", ptr(x), ptr(h), C.byref(net), int(S), ptr(ccw), ptr(ccn), ptr(z), ptr(zrev), ptr(jac),
                   ptr(logdet), ptr(saved), R, d, ptr(ws), nbytes, stream_ptr())
         ctx.lw_passes = lw_passes if (lw_passes is not None and train) else None
-        ctx.fused_bwd = fused_bwd
+        ctx.tc3 = tc3
         _count(2)
         ctx.saved_acts = saved
         ctx.save_for_backward(x, h, jac, *weights, *biases)
@@ -1104,9 +1104,11 @@ class UmnnFn(torch.autograd.Function):
         for l in range(n):
             grads.dW[l] = dWs[l].data_ptr()
             grads.db[l] = dbs[l].data_ptr()
-        if ctx.lw_passes is not None and ctx.fused_bwd:
+        if ctx.tc3:
             # dgrad chain fused on the tensor cores (tc_umnn3.cu), then the resident weight-gradient GEMMs
             nbytes = lib().gnf_umnn_bwd_tc3_workspace_bytes(C.byref(net), R, ctx.S)
+            if nbytes == 0:
+                raise RuntimeError("libgnf: " + lib().gnf_last_error().decode())
             ws = torch.empty((nbytes + 3) // 4, device=x.device, dtype=torch.float32)
             _call("gnf_umnn_bwd_tc3", ptr(x), ptr(h), C.byref(net), ctx.S, ptr(ccw), ptr(ccn), ptr(jac), ptr(gz), ptr(gzrev),
                   ptr(gjac), ptr(glogdet), ptr(ctx.saved_acts), ptr(dx), ptr(dh), C.byref(grads), R, d, ptr(ws), nbytes, stream_ptr())
@@ -1163,45 +1165,6 @@ def umnn_invert(z, h, S, weights, biases, iters=20, lo=-20., hi=20.):
 
 def _pad32(v):
     return (v + 31) // 32 * 32
-
-
-def linear_fwd_rw(X, W, bias, relu, passes=3, want_bits=False):
-    """Y = act(X[:, :K] @ W^T + bias) on the resident-weight tensor-core kernel (tc_rw.cu).  X: [M, pad32(K)] with zero
-    padding columns; returns Y [M, pad32(N)] (padding columns 0) and, if want_bits, the ReLU bit mask [M, pad32(N)/32]."""
-    require(X, "X"), require(W, "W")
-    N, K = W.shape
-    M = X.shape[0]
-    if X.shape[1] != _pad32(K):
-        raise ValueError(f"X must have pad32(K) = {_pad32(K)} columns")
-    nbytes = lib().gnf_linear_rw_workspace_bytes(N, K)
-    if nbytes == 0:
-        raise RuntimeError("libgnf: " + lib().gnf_last_error().decode())
-    ws = torch.empty(nbytes // 4, device=X.device, dtype=torch.float32)
-    Y = torch.empty(M, _pad32(N), device=X.device, dtype=torch.float32)
-    bits = torch.empty(M, _pad32(N) // 32, device=X.device, dtype=torch.int32) if want_bits else None
-    _call("gnf_linear_fwd_rw", ptr(X), X.stride(0), ptr(W), W.stride(0), ptr(bias), ptr(Y), Y.stride(0), ptr(bits), M, N, K,
-          int(relu), int(passes), ptr(ws), nbytes, stream_ptr())
-    _count(2)
-    return (Y, bits) if want_bits else Y
-
-
-def linear_dgrad_rw(dY, W, act=None, mask_bits=None, passes=3):
-    """dX = (dY[:, :N] @ W) o relu'(.) on the resident-weight kernel.  dY: [M, pad32(N)] (zero padding); act [M, pad32(K)]
-    or mask_bits [M, pad32(K)/32] select the ReLU mask; returns dX [M, pad32(K)]."""
-    require(dY, "dY"), require(W, "W")
-    N, K = W.shape
-    M = dY.shape[0]
-    if dY.shape[1] != _pad32(N):
-        raise ValueError(f"dY must have pad32(N) = {_pad32(N)} columns")
-    nbytes = lib().gnf_linear_rw_workspace_bytes(K, N)
-    if nbytes == 0:
-        raise RuntimeError("libgnf: " + lib().gnf_last_error().decode())
-    ws = torch.empty(nbytes // 4, device=dY.device, dtype=torch.float32)
-    dX = torch.empty(M, _pad32(K), device=dY.device, dtype=torch.float32)
-    _call("gnf_linear_dgrad_rw", ptr(dY), dY.stride(0), ptr(W), W.stride(0), ptr(act), act.stride(0) if act is not None else 0,
-          ptr(mask_bits), ptr(dX), dX.stride(0), M, N, K, int(passes), ptr(ws), nbytes, stream_ptr())
-    _count(2)
-    return dX
 
 
 def linear_wgrad_rw(dY, X, N, K, passes=3):

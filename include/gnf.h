@@ -389,21 +389,6 @@ int gnf_dag_loss_bwd(const float* A, int d, const float* t, const float* lambd, 
                      const float* l1_weight, const float* gout, float* dA, float* dt, gnf_stream_t stream);
 
 
-/* Resident-weight tensor-core layer GEMM (tc_rw.cu) -- the hidden x hidden layers of IntegrandNet
- * (MonotonicNormalizer.py:12-38) over all quadrature node-rows, forward and dgrad.  The layer's weights (N, K <= 160) are
- * split into TF32 hi / lo images once per call and stay resident in shared memory; the activations stream global ->
- * registers -> TMEM (no shared-memory staging), TS-form tcgen05.mma, row-owner epilogue.  passes as gnf_linear_*_tc.
- * Operand contract (what the layer-wise engine's padded planes satisfy): X / dY / Y / dX rows 32-byte aligned (leading dimensions multiples of 8), X / dY with
- * round_up(K or N, 32) readable columns whose padding is zero; Y / dX receive round_up(N or K, 32) columns per row.
- * bits_out (nullable): ReLU bit mask of Y, [M][round_up(N,32)/32] words; mask_bits (nullable, same layout) or act select
- * the ReLU mask of dgrad.  work: gnf_linear_rw_workspace_bytes(N, K) bytes (0 = shape unsupported, see gnf_last_error). */
-size_t gnf_linear_rw_workspace_bytes(int N, int K);
-int gnf_linear_fwd_rw(const float* X, int ldx, const float* W, int ldw, const float* bias, float* Y, int ldy, uint32_t* bits_out,
-                      int M, int N, int K, int relu, int passes, void* work, size_t work_bytes, gnf_stream_t stream);
-int gnf_linear_dgrad_rw(const float* dY, int lddy, const float* W, int ldw, const float* act, int ldact,
-                        const uint32_t* mask_bits, float* dX, int lddx, int M, int N, int K, int passes, void* work,
-                        size_t work_bytes, gnf_stream_t stream);
-
 /* Weight gradient of an IntegrandNet hidden layer (MonotonicNormalizer.py:12-38) over all quadrature node-rows -- the parameter
  * gradient UMNN's NeuralIntegral.backward accumulates node by node (SURVEY App. B) -- (tc_rw_wgrad.cu): dW[N,K] = dY^T X,
  * N, K <= 160, M rows.  TMEM lane =

@@ -31,17 +31,6 @@ int gnf_tc_gemm_set_trace(long long* buf);
  * resident in shared memory (every gate evaluated once per direction); 0 = functor-loader tile GEMM for every d. */
 int gnf_dag_l1_set_resident(int enable);
 
-/* Measurement switch: 0 routes the layer-wise engine's hidden GEMMs to the generic tensor-core engine (gnf_linear_*_tc)
- * instead of the resident-weight kernels below; 3 keeps forward/dgrad resident but runs wgrad on the generic engine.  Default 1. */
-int gnf_umnn_lw_set_rw(int enable);
-
-/* Measurement: later resident-weight GEMM launches write SM-clock stamps of CTA 0 into buf (4 x 256 int64, device; rows:
- * MMA issuer, loader of even chunks, loader of odd chunks, epilogue).  NULL disables. */
-int gnf_linear_rw_set_trace(long long* buf);
-
-/* Measurement: bit0 skips the kernel's global stores, bit1 its global loads, bit2 its MMAs (results are then garbage). */
-int gnf_linear_rw_set_debug(int bits);
-
 /* Measurement: later gnf_linear_wgrad_rw launches write SM-clock stamps of CTA 0 into buf (3 x 256 int64, device; rows: MMA
  * issuer, first stager thread, first loader thread).  NULL disables. */
 int gnf_linear_wgrad_rw_set_trace(long long* buf);

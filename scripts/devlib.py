@@ -16,9 +16,6 @@ DEV_PROTOS = {
     "gnf_tc_gemm_set_fold": ([_I], C.c_int),
     "gnf_tc_gemm_set_trace": ([_P], C.c_int),
     "gnf_dag_l1_set_resident": ([_I], C.c_int),
-    "gnf_umnn_lw_set_rw": ([_I], C.c_int),
-    "gnf_linear_rw_set_trace": ([_P], C.c_int),
-    "gnf_linear_rw_set_debug": ([_I], C.c_int),
     "gnf_linear_wgrad_rw_set_trace": ([_P], C.c_int),
     "gnf_tc_probe": ([_I, _I, _P, _P], C.c_int),
     "gnf_tc_set_trace": ([_P], C.c_int),

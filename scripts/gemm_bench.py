@@ -28,20 +28,6 @@ for (M, N, K) in [(138600, 160, 160), (138600, 152, 152), (6300, 632, 632), (630
     tt = t(lambda: torch.relu(X @ W.t() + b))
     print(f"      torch fp32 (cuBLAS) fwd {tt*1e3:.0f}us {fl/tt/1e9:.0f}TF")
 
-print("resident-weight kernel (tc_rw.cu), padded operands")
-for (M, N, K) in [(138600, 150, 150), (258300, 150, 150), (1419264, 150, 150), (150000, 100, 100)]:
-    NP, KP = (N + 31) // 32 * 32, (K + 31) // 32 * 32
-    X = torch.zeros(M, KP, device="cuda"); X[:, :K] = torch.randn(M, K, device="cuda")
-    W = torch.randn(N, K, device="cuda") / K ** .5; b = torch.randn(N, device="cuda")
-    dY = torch.zeros(M, NP, device="cuda"); dY[:, :N] = torch.randn(M, N, device="cuda")
-    fl = 2. * M * N * K
-    row = f"M={M} N={N} K={K}:"
-    for passes in (1, 3):
-        a = t(lambda: G.ops.linear_fwd_rw(X, W, b, relu=True, passes=passes, want_bits=True))
-        c = t(lambda: G.ops.linear_dgrad_rw(dY, W, act=X, passes=passes))
-        row += f"  passes={passes}: fwd {a*1e3:.0f}us {fl/a/1e9:.0f}TF {M*(NP+KP)*4/a/1e6:.0f}GB/s  dgrad(act mask) {c*1e3:.0f}us {fl/c/1e9:.0f}TF |"
-    print(row)
-
 print("resident wgrad kernel (tc_rw_wgrad.cu)")
 for (M, N, K) in [(138600, 150, 150), (1419264, 150, 150), (150000, 100, 100)]:
     NPn, KP = (N + 31) // 32 * 32, (K + 31) // 32 * 32

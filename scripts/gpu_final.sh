@@ -19,7 +19,7 @@ echo "== ncu launch list"
 timeout 900 ncu --metrics gpu__time_duration.sum --clock-control none -c 1200 --csv --log-file $OUT/launches.csv \
   python bench.py --steps 2 --warmup 3 --no-cpu-baseline --no-eval --cuda-graph off > $OUT/ncu_launches.log 2>&1
 echo "== ncu full: tcgen05 GEMM kernels"
-timeout 900 ncu --set full --clock-control none --import-source on -k regex:"tc_gemm|rw_gemm|rw_wgrad_kernel" -s 36 -c 12 -o $OUT/prof_gemms -f \
+timeout 900 ncu --set full --clock-control none --import-source on -k regex:"tc_gemm|rw_wgrad_kernel" -s 36 -c 12 -o $OUT/prof_gemms -f \
   python bench.py --steps 2 --warmup 3 --no-cpu-baseline --no-eval --cuda-graph off > $OUT/ncu_gemms.log 2>&1
 tail -2 $OUT/ncu_gemms.log
 ls -la $OUT

@@ -266,100 +266,12 @@ def test_umnn_layerwise_auto_engine_selection(umnn_engine):
 
 
 # ---------------------------------------------------------------------------------------------------------------
-# resident-weight layer GEMM (tc_rw.cu): the hidden layers of the layer-wise UMNN engine
+# resident weight-gradient kernel (tc_rw_wgrad.cu): the hidden-layer weight gradients of the fused UMNN backward
 # ---------------------------------------------------------------------------------------------------------------
 def _padded(t, cols):
     out = torch.zeros(t.shape[0], cols, device=t.device, dtype=t.dtype)
     out[:, :t.shape[1]] = t
     return out
-
-
-RW_SHAPES = [(1000, 150, 150), (128, 160, 100), (4133, 100, 100), (77, 30, 150), (300, 150, 31), (20000, 150, 150)]
-
-
-@pytest.mark.parametrize("M_,N,K", RW_SHAPES)
-def test_rw_gemm_exact_on_small_integers(M_, N, K):
-    g = torch.Generator(device="cuda").manual_seed(M_ + N + K)
-    X = torch.randint(-8, 9, (M_, K), device="cuda", generator=g).float()
-    W = torch.randint(-8, 9, (N, K), device="cuda", generator=g).float()
-    b = torch.randint(-8, 9, (N,), device="cuda", generator=g).float()
-    NP, KP = (N + 31) // 32 * 32, (K + 31) // 32 * 32
-    for passes in (1, 3):
-        Y, bits = G.ops.linear_fwd_rw(_padded(X, KP), W, b, relu=True, passes=passes, want_bits=True)
-        ref = torch.relu(X @ W.t() + b)
-        assert torch.equal(Y[:, :N], ref), f"fwd passes={passes}: max err {float((Y[:, :N] - ref).abs().max())}"
-        assert float(Y[:, N:].abs().max()) == 0. if NP > N else True
-        # bit mask of the output
-        cols = torch.arange(NP, device="cuda")
-        got = ((bits.long().unsqueeze(2) >> (cols % 32).view(1, NP // 32, 32)) & 1).view(M_, NP)[:, :N].bool()
-        assert torch.equal(got, ref > 0)
-        dY = torch.randint(-8, 9, (M_, N), device="cuda", generator=g).float()
-        act = _padded(torch.randint(-3, 4, (M_, K), device="cuda", generator=g).float(), KP)
-        dX = G.ops.linear_dgrad_rw(_padded(dY, NP), W, act=act, passes=passes)
-        refd = (dY @ W) * (act[:, :K] > 0)
-        assert torch.equal(dX[:, :K], refd), f"dgrad passes={passes}: max err {float((dX[:, :K] - refd).abs().max())}"
-        # the same mask as bits
-        mb = torch.zeros(M_, KP // 32, dtype=torch.int64, device="cuda")
-        on = (act > 0).long().view(M_, KP // 32, 32)
-        mb = (on << torch.arange(32, device="cuda").view(1, 1, 32)).sum(2)
-        mb = torch.where(mb >= 2 ** 31, mb - 2 ** 32, mb).to(torch.int32)
-        dX2 = G.ops.linear_dgrad_rw(_padded(dY, NP), W, mask_bits=mb, passes=passes)
-        assert torch.equal(dX2[:, :K], refd)
-
-
-@pytest.mark.parametrize("M_,N,K", RW_SHAPES)
-def test_rw_gemm_3xtf32_is_fp32_equivalent(M_, N, K):
-    g = torch.Generator(device="cuda").manual_seed(7 * M_ + N)
-    X = torch.randn(M_, K, device="cuda", generator=g)
-    W = torch.randn(N, K, device="cuda", generator=g) / K ** .5
-    b = torch.randn(N, device="cuda", generator=g)
-    KP = (K + 31) // 32 * 32
-    Y = G.ops.linear_fwd_rw(_padded(X, KP), W, b, relu=False, passes=3)[:, :N]
-    ref64 = X.double() @ W.double().t() + b.double()
-    err = float((Y.double() - ref64).abs().max() / ref64.abs().max())
-    err32 = float(((X @ W.t() + b).double() - ref64).abs().max() / ref64.abs().max())
-    assert err < max(2e-6, 4 * err32), (err, err32)
-    Y1 = G.ops.linear_fwd_rw(_padded(X, KP), W, b, relu=False, passes=1)[:, :N]
-    assert float((Y1.double() - ref64).abs().max() / ref64.abs().max()) < 3e-3
-
-
-def test_rw_gemm_unsupported_width_is_loud():
-    X = torch.zeros(8, 224, device="cuda")
-    W = torch.zeros(200, 200, device="cuda")
-    with pytest.raises(RuntimeError):
-        G.ops.linear_fwd_rw(X, W, None, relu=True)
-
-
-def test_umnn_layerwise_rw_and_generic_engines_agree(umnn_engine):
-    """Same layer-wise step through the resident-weight kernel and through the generic tensor-core engine."""
-    import ctypes as C
-    import os
-    import model_vs_oracle as M
-    dev_so = os.path.join(os.path.dirname(G._lib.LIB_PATH), "libgnf_sm100_dev.so")
-    assert os.path.isfile(dev_so), "engine override is a development-build knob: __graft_entry__.build() builds libgnf_sm100_dev.so"
-    devlib = C.CDLL(dev_so)          # the knob is process-global state of THAT library: route the package through it for this test
-    product = G._lib._lib
-    G._lib._lib = G._lib._bind(devlib)   # AttributeError: a stale development build (rebuild with build.py --dev)
-    umnn_engine("layerwise", "tf32x3")
-    model = M.build(M.CONFIGS["cfg4"], "cuda")
-    parity.set_modes(model, dict(stoch_gate=False))
-    x = torch.randn(64, 63, device="cuda", generator=torch.Generator(device="cuda").manual_seed(5))
-    outs = []
-    try:
-        for rw in (1, 0, 3):
-            devlib.gnf_umnn_lw_set_rw(rw)
-            model.zero_grad()
-            z, jac = model(x)
-            model.loss(z, jac).backward()
-            outs.append((z.detach().clone(), {k: p.grad.clone() for k, p in model.named_parameters() if p.grad is not None}))
-    finally:
-        devlib.gnf_umnn_lw_set_rw(1)
-        G._lib._lib = product
-    for other in (1, 2):
-        assert float((outs[0][0] - outs[other][0]).abs().max()) < 1e-4
-        for k in outs[0][1]:
-            a, b = outs[0][1][k], outs[other][1][k]
-            assert float((a - b).norm() / b.norm().clamp_min(1e-20)) < 2e-4, k
 
 
 @pytest.mark.parametrize("M_,N,K", [(1000, 150, 150), (32, 160, 160), (4133, 100, 100), (77, 30, 150), (300, 150, 31), (40000, 150, 150),

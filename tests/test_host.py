@@ -205,6 +205,33 @@ def test_tensor_core_gemm_plan_fills_the_last_round_of_work_items():
     assert lib.gnf_tc_gemm_plan(0, 1, 1, 3, 0, C.byref(bn), C.byref(sp)) != 0
 
 
+def test_fused_umnn_backward_takes_every_net_the_fused_forward_takes():
+    """A training forward on gnf_umnn_fwd_tc3 is always followed by gnf_umnn_bwd_tc3, so at S + 1 <= 256 nodes the two workspace
+    queries accept the same integrands: 3- and 4-layer nets over hidden widths on both sides of every 32-column padding step,
+    up to 160 and one past it.  Host-only queries (the weight pointers are never read)."""
+    import ctypes as C
+    import itertools
+    import __graft_entry__
+    __graft_entry__.build()
+    lib = G._lib.load_library()
+    E, R = 5, 240
+    widths = (1, 31, 32, 33, 64, 128, 129, 152, 153, 160, 161)
+    accepted = 0
+    for hidden in itertools.chain(itertools.product(widths, repeat=2), itertools.product(widths, repeat=3)):
+        net = G._lib.MlpT()
+        dims = [1 + E, *hidden, 1]
+        net.n_layers = len(dims) - 1
+        for i, v in enumerate(dims):
+            net.dims[i] = v
+        fwd = lib.gnf_umnn_tc3_workspace_bytes(C.byref(net), R)
+        assert (fwd != 0) == (max(hidden) <= 160), hidden
+        for S in (20, 255):
+            bwd = lib.gnf_umnn_bwd_tc3_workspace_bytes(C.byref(net), R, S)
+            assert (bwd != 0) == (fwd != 0), (hidden, S, lib.gnf_last_error())
+        accepted += fwd != 0
+    assert accepted == 10 ** 2 + 10 ** 3
+
+
 # ---------------- experiment plumbing (SURVEY 8f rank 4) ----------------
 def test_reference_yaml_preset_and_driver_defaults(tmp_path):
     """A preset in the reference's YAML format (UCIExperimentsConfigurations.yml:1-14) merged over the driver's argparse defaults;
