@@ -78,12 +78,15 @@ _PROTOS = {
     "gnf_dag_l1_wgrad": ([_P, _I, _P, _P, C.POINTER(GateT), _P, _I, _I, _I, _I, _P], C.c_int),
     "gnf_dag_l1_dgrad": ([_P, _I, _P, _I, _P, _P, C.POINTER(GateT), _P, _P, _I, _I, _I, _P], C.c_int),
     "gnf_dag_l1_fwd_save": ([_P, _P, C.POINTER(GateT), _P, _I, _P, _I, _P, _I, _P, _P, _P, _I, _I, _I, _I, _P], C.c_int),
+    "gnf_dag_l1_fwd_cond": ([_P, _P, C.POINTER(GateT), _P, _I, _P, _I, _I, _P, _I, _P, _I, _P, _P, _P, _I, _I, _I, _I, _P], C.c_int),
+    "gnf_dag_l1_bias_sums": ([_P, _I, _P, _P, _I, _I, _I, _I, _I, _P], C.c_int),
     "gnf_dag_l1_wgrad_saved": ([_P, _I, _P, _P, _I, _I, _I, _I, _P], C.c_int),
     "gnf_dag_l1_dgrad_saved": ([_P, _I, _P, _I, _P, _P, _P, _P, _I, _I, _I, _P], C.c_int),
     "gnf_linear_fwd_splitk_workspace_bytes": ([_I, _I, _I], _SZ),
     "gnf_linear_fwd_splitk": ([_P, _I, _P, _I, _P, _P, _I, _I, _I, _I, _I, _P, _SZ, _P], C.c_int),
     "gnf_dag_bias_table_ld": ([_P, _I, _P, _P, _I, _I, _I, _I, _P], C.c_int),
     "gnf_linear_fwd_tc_ps_tb": ([_P, _I, _P, _P, _I, _P, _I, _I, _P, _I, _I, _I, _I, _I, _P], C.c_int),
+    "gnf_linear_fwd_tc_cond": ([_P, _I, _P, _P, _I, _P, _I, _I, _P, _I, _I, _P, _I, _I, _I, _I, _I, _I, _P], C.c_int),
     "gnf_dag_gate_planes": ([_P, _P, C.POINTER(GateT), _P, _P, _P, _I, _I, _P], C.c_int),
     "gnf_dag_l1_reduce_saved": ([_P, _P, _P, _P, _P, _I, _I, _P], C.c_int),
     "gnf_nll_loss_work_floats": ([_I], _SZ),

@@ -30,6 +30,17 @@ def _linear_stack(sizes):
     return nn.Sequential(*layers)
 
 
+def _check_context(context, B, cond_in, who):
+    """A conditional conditioner's context: [B, cond_in], CUDA, fp32, contiguous (ValueError for a missing or misshapen one,
+    TypeError for the rest, like every op)."""
+    if context is None:
+        raise ValueError(f"{who}: built with cond_in={cond_in}, forward needs a [B, {cond_in}] context")
+    L.require(context, "context")
+    if tuple(context.shape) != (B, cond_in):
+        raise ValueError(f"{who}: context must be [B, cond_in] = [{B}, {cond_in}], got {tuple(context.shape)}")
+    return context
+
+
 def _stack_params(net):
     """[W0, b0, W1, b1, ...] of the nn.Linear members of an nn.Sequential, rejecting anything that the
     fused kernels do not implement (only Linear/ReLU alternation)."""
@@ -73,6 +84,7 @@ class DAGConditioner(Conditioner):
         self.stoch_gate = True
         self.noise_gate = False
         in_net = in_size * 2 if hot_encoding else in_size
+        self.cond_in = cond_in
         self._module_embedding = isinstance(hidden, nn.Module)
         if self._module_embedding:
             # an arbitrary embedding module (the reference's image flows pass MNISTCNN / CIFAR10CNN, DAGConditioner.py:38-39):
@@ -178,7 +190,12 @@ class DAGConditioner(Conditioner):
                             offset=(self._noise_rank << 40) + self._noise_calls)
 
     def forward(self, x, context=None):
-        # context is accepted and ignored exactly like the reference (quirk Q8)
+        """h [B, d, H].  With cond_in = c > 0, context [B, c] joins layer 1's input: the row for sample b, variable i is
+        [e[b,i,:] | onehot(i) (hot_encoding) | context[b,:]], the in_net + cond_in columns DAGMLP's first Linear is built with
+        (see ops.DagMlpFn).  With cond_in = 0, or an nn.Module embedding, a context is accepted and ignored like the reference
+        (quirk Q8)."""
+        if self.cond_in > 0 and not self._module_embedding:
+            _check_context(context, x.shape[0], self.cond_in, "DAGConditioner")
         gate = self._gate_spec(x)
         self._last_gate = gate          # lets tests dump the Philox draws this forward used
         if self._module_embedding:
@@ -187,7 +204,10 @@ class DAGConditioner(Conditioner):
             if self.hot_encoding:       # DAGConditioner.py:155-166: the one-hot block goes in front of the embedding net
                 e = torch.cat((e, torch.eye(d, device=e.device, dtype=e.dtype).repeat(B, 1)), 1)
             return self.embedding_net(e).view(B, d, -1)
-        return ops.DagMlpFn.apply(x.contiguous(), self.A, gate, self.hot_encoding, *_stack_params(self.embedding_net.net))
+        params = _stack_params(self.embedding_net.net)
+        if self.cond_in > 0:
+            params.append(context)
+        return ops.DagMlpFn.apply(x.contiguous(), self.A, gate, self.hot_encoding, *params)
 
     def _alpha_host(self):
         # alpha is a registered buffer (checkpoint compatibility) but only ever holds 1/d; cache its host value
@@ -500,10 +520,18 @@ class CouplingConditioner(Conditioner):
         self.out_size = out_size
         self.cond_size = int(in_size / 2)
         self.indep_size = in_size - self.cond_size
+        self.cond_in = cond_in
         self.embeding_net = CouplingMLP(in_size, hidden, out_size, cond_in)
         self.constants = nn.Parameter(torch.randn(self.indep_size, out_size))
 
     def forward(self, x, context=None):
+        """With cond_in = c > 0 the embedding net takes cat(x[:, :indep], context) (its indep + cond_in inputs); with c = 0 a
+        context is concatenated and sliced away again, like the reference (quirk Q8)."""
+        if self.cond_in > 0:
+            _check_context(context, x.shape[0], self.cond_in, "CouplingConditioner")
+            inp = torch.cat((x[:, :self.indep_size], context), 1)
+            h2 = ops.MlpFn.apply(inp, inp.shape[1], *_stack_params(self.embeding_net.net))
+            return _CouplingAssemble.apply(self.constants, h2, x.shape[0], self.in_size, self.indep_size, self.out_size)
         if context is not None:
             x = torch.cat((x, context), 1)                  # then sliced away again, like the reference (quirk Q8)
         x = x.contiguous()

@@ -26,6 +26,8 @@ def build_from_spec(spec, device=None, seed=None):
     if seed is not None:
         torch.manual_seed(seed)
     cargs = {"in_size": spec["d"], "hidden": list(spec["hidden"]), "out_size": spec["out"]}
+    if spec.get("cond_in", 0):
+        cargs["cond_in"] = spec["cond_in"]          # conditional flow: every forward takes a [B, cond_in] context
     if spec["cond"] == "DAG":
         cargs.update(l1=spec.get("l1", 0.), gumble_T=spec.get("gumble_T", 1.), nb_epoch_update=10,
                      hot_encoding=spec.get("hot_encoding", False))

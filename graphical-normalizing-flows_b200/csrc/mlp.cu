@@ -132,6 +132,30 @@ struct EpiDagDgrad {  // ebar[m,j] -> dx[b,j] += ebar*de/dx ; dP[i,j] += ebar*de
   }
 };
 
+// Layer 1 of a conditional flow on the tile GEMM: Y = act(acc + T[m % period, n] + U[m / group, n]), the bias table plus the
+// per-sample context term (EpiBiasAct, which every FFMA linear layer shares, stays without the second term)
+struct EpiBiasCtxAct {
+  float* Y; int ldy; const float* T; int ldt; int period; const float* U; int ldu; int group; int relu;
+  __device__ __forceinline__ void operator()(int m, int n, const float* v, int nv) const {
+    float* y = Y + (size_t)m * ldy + n;
+    const float* tp = T + (size_t)(period > 1 ? (m % period) : 0) * ldt + n;
+    const float* up = U + (size_t)(m / group) * ldu + n;
+    float o[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      float r = v[j];
+      if (j < nv) r += __ldg(tp + j) + __ldg(up + j);
+      if (relu) r = fmaxf(r, 0.f);
+      o[j] = r;
+    }
+    if (nv == 4 && (reinterpret_cast<uintptr_t>(y) & 15) == 0) {
+      *reinterpret_cast<float4*>(y) = make_float4(o[0], o[1], o[2], o[3]);
+    } else {
+      for (int j = 0; j < nv; ++j) y[j] = o[j];
+    }
+  }
+};
+
 // ------------------------------------------------------------------------------------------------
 // Layer 1 of narrow DAG flows (d <= 64): gate tile resident in shared memory
 // ------------------------------------------------------------------------------------------------
@@ -162,9 +186,11 @@ constexpr size_t kDagFwdSmem = (size_t)(kDagFwdBM + kDagFwdBN) * kDagLDK * sizeo
 // transcendentals + divisions, ~300 instructions) was most of each of the three kernels (see above), now it runs once per step.
 struct GatePlanes { float* E; float* DX; float* DP; };
 
-template <bool kSave>
+// kCond (conditional flows): row m also adds its sample's context term U[m / d, :] (U = context W1[:, in_net:]^T, row stride ldu)
+template <bool kSave, bool kCond>
 __global__ void __launch_bounds__(kDagFwdThreads, 2) dag_l1_fwd_kernel(GateCtx g, GatePlanes sv, const float* __restrict__ W1, int ldw, const float* __restrict__ T,
-                                                                    int bias_ld, int period, int relu, float* __restrict__ Y, int ldy, int M, int N) {
+                                                                    int bias_ld, int period, const float* __restrict__ U, int ldu, int relu,
+                                                                    float* __restrict__ Y, int ldy, int M, int N) {
   GNF_SMEM(float, smem);
   float* Es = smem;                              // [BM][LDK]   Es[m][j]
   float* Ws = smem + kDagFwdBM * kDagLDK;        // [BN][LDK]   Ws[n][k]
@@ -200,10 +226,12 @@ __global__ void __launch_bounds__(kDagFwdThreads, 2) dag_l1_fwd_kernel(GateCtx g
   }
   const int tx = t % 32, ty = t / 32;            // lane = column residue, warp = group of 4 rows
   const float* brow[4];                          // bias-table row of each of the thread's rows (clamped for rows >= M)
+  const float* urow[4];                          // ... and its sample's context-term row (kCond)
 #pragma unroll
   for (int i = 0; i < 4; ++i) {
     const int m = (m0 + ty * 4 + i < M) ? m0 + ty * 4 + i : M - 1;
     brow[i] = T + (size_t)(period > 1 ? (m % period) : 0) * bias_ld;
+    urow[i] = kCond ? U + (size_t)(m / d) * ldu : nullptr;
   }
   for (int n0 = 0; n0 < N; n0 += kDagFwdBN) {
 #pragma unroll
@@ -222,6 +250,7 @@ __global__ void __launch_bounds__(kDagFwdThreads, 2) dag_l1_fwd_kernel(GateCtx g
       for (int c = 0; c < 4; ++c) {
         const int n = n0 + tx + 32 * c;
         acc[i][c] = T ? __ldg(brow[i] + (n < N ? n : N - 1)) : 0.f;
+        if (kCond) acc[i][c] += __ldg(urow[i] + (n < N ? n : N - 1));
       }
 #pragma unroll 2
     for (int k = 0; k < kDagKP; k += 4) {
@@ -252,6 +281,13 @@ __global__ void __launch_bounds__(kDagFwdThreads, 2) dag_l1_fwd_kernel(GateCtx g
     }
     __syncthreads();                             // Ws is overwritten by the next N tile
   }
+}
+
+static void launch_dag_l1_fwd(bool save, bool cond, const GateCtx& g, GatePlanes sv, const float* W1, int ldw, const float* T, int bias_ld, int period,
+                              const float* U, int ldu, int relu, float* Y, int ldy, int M, int N, cudaStream_t s) {
+  auto kern = save ? (cond ? dag_l1_fwd_kernel<true, true> : dag_l1_fwd_kernel<true, false>)
+                   : (cond ? dag_l1_fwd_kernel<false, true> : dag_l1_fwd_kernel<false, false>);
+  GNF_LAUNCH(kern, ceil_div(M, kDagFwdBM), kDagFwdThreads, kDagFwdSmem, s, g, sv, W1, ldw, T, bias_ld, period, U, ldu, relu, Y, ldy, M, N);
 }
 
 // Weight gradient: dW1[n, j] += sum_{m in the CTA's 64 rows} dY[m, n] e[m, j].  CTA = 64 rows of the reduction, 256 threads
@@ -700,6 +736,40 @@ __global__ void dag_dump_noise_kernel(GateCtx g, float* n1, float* n2, size_t n)
   }
 }
 
+// The two sums of layer 1's pre-activation cotangent of a conditional DAG flow, from one read of it (M = B d rows, row stride ldd):
+//   dT[m % period, n] += delta[m, n]   (the bias table's gradient; period = d or 1)      S[m / d, n] += delta[m, n]   (per sample)
+// Thread = one column n; block = (256 columns, kSumB samples, a slice of the variables i); dT and S are zeroed first and take atomics.
+constexpr int kSumB = 8;
+__global__ void __launch_bounds__(256) dag_l1_bias_sums_kernel(const float* __restrict__ delta, int ldd, float* __restrict__ dT, float* __restrict__ S,
+                                                               int lds, int B, int d, int N, int period, int i_per) {
+  const int n = blockIdx.x * blockDim.x + threadIdx.x;
+  const int b0 = blockIdx.y * kSumB, i0 = blockIdx.z * i_per, i1 = i0 + i_per < d ? i0 + i_per : d;
+  if (n >= N) return;
+  float s[kSumB];
+#pragma unroll
+  for (int u = 0; u < kSumB; ++u) s[u] = 0.f;
+  float tsum = 0.f;
+  for (int i = i0; i < i1; ++i) {
+    float v[kSumB];
+#pragma unroll
+    for (int u = 0; u < kSumB; ++u) {          // kSumB independent loads in flight (rows of samples past B are clamped, then dropped)
+      const int b = b0 + u < B ? b0 + u : B - 1;
+      v[u] = __ldg(delta + ((size_t)b * d + i) * ldd + n);
+    }
+    float t = 0.f;
+#pragma unroll
+    for (int u = 0; u < kSumB; ++u) {
+      if (b0 + u < B) { s[u] += v[u]; t += v[u]; }
+    }
+    if (period > 1) atomicAdd(dT + (size_t)i * N + n, t);
+    else tsum += t;
+  }
+  if (period == 1) atomicAdd(dT + n, tsum);
+#pragma unroll
+  for (int u = 0; u < kSumB; ++u)
+    if (b0 + u < B) atomicAdd(S + (size_t)(b0 + u) * lds + n, s[u]);
+}
+
 static inline int ew_blocks(size_t n) {
   size_t b = (n + 255) / 256;
   if (b > (size_t)8 * kNumSMs) b = (size_t)8 * kNumSMs;
@@ -865,13 +935,52 @@ int gnf_dag_l1_fwd(const float* x, const float* P, const gnf_gate_t* gate, const
   EpiBiasAct epi{Y, ldy, T, N, bias_period < 1 ? 1 : bias_period, relu};
   const int M = B * d;
   if (d <= kDagMaxD && g_dag_l1_resident) {
-    GNF_LAUNCH(dag_l1_fwd_kernel<false>, ceil_div(M, kDagFwdBM), kDagFwdThreads, kDagFwdSmem, s, g, GatePlanes{nullptr, nullptr, nullptr}, W1, ldw, T, N,
-               bias_period < 1 ? 1 : bias_period, relu, Y, ldy, M, N);
+    launch_dag_l1_fwd(false, false, g, GatePlanes{nullptr, nullptr, nullptr}, W1, ldw, T, N, bias_period < 1 ? 1 : bias_period, nullptr, 0, relu, Y, ldy, M, N, s);
     return check_launch("gnf_dag_l1_fwd");
   }
   if (d >= kGateInlineMinD) launch_gemm_auto(LoadDagA<true>{g}, bl, epi, M, N, d, false, s);
   else launch_gemm_auto(LoadDagA<false>{g}, bl, epi, M, N, d, false, s);
   return check_launch("gnf_dag_l1_fwd");
+}
+
+int gnf_dag_l1_fwd_cond(const float* x, const float* P, const gnf_gate_t* gate, const float* W1, int ldw, const float* T, int ldt, int bias_period,
+                        const float* U, int ldu, float* Y, int ldy, float* E, float* DX, float* DP, int B, int d, int N, int relu, gnf_stream_t stream) {
+  if (!x || !P || !W1 || !T || !U || !Y || B < 0 || d <= 0 || N <= 0 || ldw < d || ldt < N || ldu < N || ldy < N || bias_period < 1 ||
+      (bias_period > 1 && bias_period != d))
+    return fail(GNF_ERR_INVALID, "gnf_dag_l1_fwd_cond: bad arguments");
+  const bool save = E || DX || DP;
+  if (save && (!E || !DX || !DP)) return fail(GNF_ERR_INVALID, "gnf_dag_l1_fwd_cond: the gate planes go together (all three or none)");
+  if (save && d > kDagMaxD) return fail(GNF_ERR_UNSUPPORTED, "gnf_dag_l1_fwd_cond: gate planes for d <= 64 only");
+  if (save && ((reinterpret_cast<uintptr_t>(DX) | reinterpret_cast<uintptr_t>(DP)) & 15) != 0) return fail(GNF_ERR_INVALID, "gnf_dag_l1_fwd_cond: planes must be 16-byte aligned");
+  GateCtx g;
+  if (int e = make_gate(&g, x, P, gate, d)) return e;
+  if (B == 0) return 0;
+  cudaStream_t s = (cudaStream_t)stream;
+  const int M = B * d;
+  if (save || (d <= kDagMaxD && g_dag_l1_resident)) {
+    launch_dag_l1_fwd(save, true, g, GatePlanes{E, DX, DP}, W1, ldw, T, ldt, bias_period, U, ldu, relu, Y, ldy, M, N, s);
+    return check_launch("gnf_dag_l1_fwd_cond");
+  }
+  LoadWeightT bl{W1, ldw};
+  EpiBiasCtxAct epi{Y, ldy, T, ldt, bias_period, U, ldu, d, relu};
+  if (d >= kGateInlineMinD) launch_gemm_auto(LoadDagA<true>{g}, bl, epi, M, N, d, false, s);
+  else launch_gemm_auto(LoadDagA<false>{g}, bl, epi, M, N, d, false, s);
+  return check_launch("gnf_dag_l1_fwd_cond");
+}
+
+int gnf_dag_l1_bias_sums(const float* delta, int ldd, float* dT, float* S, int lds, int B, int d, int N, int period, gnf_stream_t stream) {
+  if (!delta || !dT || !S || B < 0 || d <= 0 || N <= 0 || ldd < N || lds < N || (period != 1 && period != d))
+    return fail(GNF_ERR_INVALID, "gnf_dag_l1_bias_sums: bad arguments");
+  cudaStream_t s = (cudaStream_t)stream;
+  cudaMemsetAsync(dT, 0, (size_t)period * N * sizeof(float), s);
+  zero2d(S, lds, B, N, s);
+  if (B == 0) return check_launch("gnf_dag_l1_bias_sums");
+  const int cblocks = ceil_div(N, 256), bblocks = ceil_div(B, kSumB);
+  int isplit = ceil_div(4 * kNumSMs, cblocks * bblocks);
+  if (isplit > d) isplit = d;
+  const int i_per = ceil_div(d, isplit);
+  GNF_LAUNCH(dag_l1_bias_sums_kernel, dim3(cblocks, bblocks, ceil_div(d, i_per)), 256, 0, s, delta, ldd, dT, S, lds, B, d, N, period, i_per);
+  return check_launch("gnf_dag_l1_bias_sums");
 }
 
 int gnf_dag_l1_wgrad(const float* dY, int lddy, const float* x, const float* P, const gnf_gate_t* gate, float* dW1,
@@ -1000,8 +1109,8 @@ int gnf_dag_l1_fwd_save(const float* x, const float* P, const gnf_gate_t* gate, 
   if (int e = make_gate(&g, x, P, gate, d)) return e;
   if (B == 0) return 0;
   const int M = B * d;
-  GNF_LAUNCH(dag_l1_fwd_kernel<true>, ceil_div(M, kDagFwdBM), kDagFwdThreads, kDagFwdSmem, (cudaStream_t)stream, g, GatePlanes{E, DX, DP}, W1, ldw, T, N,
-             bias_period < 1 ? 1 : bias_period, relu, Y, ldy, M, N);
+  launch_dag_l1_fwd(true, false, g, GatePlanes{E, DX, DP}, W1, ldw, T, N, bias_period < 1 ? 1 : bias_period, nullptr, 0, relu, Y, ldy, M, N,
+                    (cudaStream_t)stream);
   return check_launch("gnf_dag_l1_fwd_save");
 }
 

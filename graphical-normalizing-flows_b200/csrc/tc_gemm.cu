@@ -172,6 +172,8 @@ __device__ __forceinline__ void trace_stamp(long long* trace, int role, long lon
   if (trace && blockIdx.x == 0 && i < kTraceLen) trace[role * kTraceLen + i] = clock64();
 }
 
+// kRowTerm: the epilogue also adds p.rowterm (a per-row-group term, see TcGemmParams) next to the periodic bias table
+template <bool kRowTerm>
 __global__ void __launch_bounds__(kGemmThreads) tc_gemm_kernel(TcGemmParams p, int vecA, int vecB, const __grid_constant__ CUtensorMap tmA,
                                                                const __grid_constant__ CUtensorMap tmB, const __grid_constant__ CUtensorMap tmBlo) {
   using namespace tc;
@@ -356,9 +358,9 @@ __global__ void __launch_bounds__(kGemmThreads) tc_gemm_kernel(TcGemmParams p, i
     //   bit_mask: the ReLU mask as one bit per element: the row owner holds its row's words
     const bool bit_mask = p.epi == TCG_EPI_MASK && p.mask_bits != nullptr;
     const bool aux_mask = p.epi == TCG_EPI_MASK && p.act != nullptr && !bit_mask;
-    const bool aux_bias = p.epi == TCG_EPI_BIAS_ACT && p.bias != nullptr && p.bias_period > 1;
+    const bool aux_bias = p.epi == TCG_EPI_BIAS_ACT && p.bias != nullptr && (p.bias_period > 1 || kRowTerm);
     const bool aux_tile = aux_mask || aux_bias;
-    const bool bias_row = p.epi == TCG_EPI_BIAS_ACT && p.bias != nullptr && p.bias_period <= 1;
+    const bool bias_row = p.epi == TCG_EPI_BIAS_ACT && p.bias != nullptr && p.bias_period <= 1 && !kRowTerm;
     int gcount = 0, tcount = 0;
     for (long long w = blockIdx.x; w < total; w += gridDim.x, ++tcount) {
       const int tm = (int)(w % tiles_m), tn = (int)((w / tiles_m) % tiles_n), sp = (int)(w / ((long long)tiles_m * tiles_n));
@@ -419,6 +421,18 @@ __global__ void __launch_bounds__(kGemmThreads) tc_gemm_kernel(TcGemmParams p, i
                 if (n + piece + 1 < p.N) v.y = __ldg(ap + 1);
                 if (n + piece + 2 < p.N) v.z = __ldg(ap + 2);
                 if (n + piece + 3 < p.N) v.w = __ldg(ap + 3);
+              }
+              if (kRowTerm) {                            // + the row group's term (bias tables only: kRowTerm implies TCG_EPI_BIAS_ACT)
+                const float* up = p.rowterm + (long long)(mr / p.rt_group) * p.rt_ld + n + piece;
+                if (p.rt_vec && n + piece + 4 <= p.N) {
+                  const float4 u = __ldg(reinterpret_cast<const float4*>(up));
+                  v.x += u.x; v.y += u.y; v.z += u.z; v.w += u.w;
+                } else {
+                  v.x += __ldg(up);
+                  if (n + piece + 1 < p.N) v.y += __ldg(up + 1);
+                  if (n + piece + 2 < p.N) v.z += __ldg(up + 2);
+                  if (n + piece + 3 < p.N) v.w += __ldg(up + 3);
+                }
               }
             }
             a[i] = v;
@@ -677,6 +691,7 @@ constexpr uint32_t kG2StageBytes = 3u * kG2TileBytes;             // raw A, B_hi
 constexpr int kG2EpiStageFloats = 32 * 32;
 constexpr int kG2Parts = 2, kG2Ring = 4;   // partial accumulators of 128 TMEM columns, then A buffers of (hi 32 + lo 32) columns
 
+template <bool kRowTerm>     // as tc_gemm_kernel's
 __global__ void __launch_bounds__(kG2Threads, 1) tc_gemm2_kernel(TcGemmParams p, const __grid_constant__ CUtensorMap tmA,
                                                                  const __grid_constant__ CUtensorMap tmB, const __grid_constant__ CUtensorMap tmBlo) {
   using namespace tc;
@@ -824,7 +839,7 @@ __global__ void __launch_bounds__(kG2Threads, 1) tc_gemm2_kernel(TcGemmParams p,
     float* stage = epi_stage + warp * kG2EpiStageFloats;
     const int sub = lane >> 3, piece = lane & 7;
     const bool mask = p.epi == TCG_EPI_MASK && p.act != nullptr;          // a dgrad without a ReLU behind it (act == NULL) stores the plain product
-    const bool table = !mask && p.bias != nullptr && p.bias_period > 1;   // periodic bias table (DAG layer 1: one row per variable): added on the coalesced side
+    const bool table = !mask && p.bias != nullptr && (p.bias_period > 1 || kRowTerm);   // periodic bias table (DAG layer 1: one row per variable): added on the coalesced side
     const int ngroups = (nchunks + fold - 1) / fold;
     int gcount = 0;
     for (int w = blockIdx.x; w < total; w += gridDim.x) {
@@ -926,6 +941,15 @@ __global__ void __launch_bounds__(kG2Threads, 1) tc_gemm2_kernel(TcGemmParams p,
               tb[i] = __ldg(reinterpret_cast<const float4*>(p.bias + (long long)(mc % p.bias_period) * p.bias_ld + ncl));
             }
           }
+          float4 tu[8];                                  // kRowTerm: the row groups' pieces, unconditional loads in flight with tb[]
+          if (kRowTerm) {
+            const int ncl = n < p.N ? n : 0;
+#pragma unroll
+            for (int i = 0; i < 8; ++i) {
+              const int m = m0 + 4 * i + sub, mc = m < p.M ? m : p.M - 1;
+              tu[i] = __ldg(reinterpret_cast<const float4*>(p.rowterm + (long long)(mc / p.rt_group) * p.rt_ld + ncl));
+            }
+          }
 #pragma unroll
           for (int i = 0; i < 8; ++i) {
             const int R = 4 * i + sub, m = m0 + R;
@@ -937,7 +961,8 @@ __global__ void __launch_bounds__(kG2Threads, 1) tc_gemm2_kernel(TcGemmParams p,
                 const uint32_t mb = mbits[c >> 5] >> (4 * i);
                 o.x = (mb & 1u) ? o.x : 0u; o.y = (mb & 2u) ? o.y : 0u; o.z = (mb & 4u) ? o.z : 0u; o.w = (mb & 8u) ? o.w : 0u;
               } else if (table) {                        // bias_ld >= round_up(N, 4) (g2_eligible): the piece is inside the padded table row,
-                const float4 b4 = tb[i];                 // whose padding columns hold anything
+                float4 b4 = tb[i];                       // whose padding columns hold anything
+                if (kRowTerm) { b4.x += tu[i].x; b4.y += tu[i].y; b4.z += tu[i].z; b4.w += tu[i].w; }
                 float v0 = __uint_as_float(o.x) + b4.x, v1 = __uint_as_float(o.y) + (n + 1 < p.N ? b4.y : 0.f),
                       v2 = __uint_as_float(o.z) + (n + 2 < p.N ? b4.z : 0.f), v3 = __uint_as_float(o.w) + (n + 3 < p.N ? b4.w : 0.f);
                 if (p.relu) { v0 = fmaxf(v0, 0.f); v1 = fmaxf(v1, 0.f); v2 = fmaxf(v2, 0.f); v3 = fmaxf(v3, 0.f); }
@@ -960,7 +985,8 @@ __global__ void __launch_bounds__(kG2Threads, 1) tc_gemm2_kernel(TcGemmParams p,
 static bool g2_eligible(const TcGemmParams& p) {
   if (p.passes != 3 || !p.B_lo || p.a_src != TCG_SRC_K || p.epi == TCG_EPI_ATOMIC || p.bits_out || p.mask_bits) return false;
   if (p.epi == TCG_EPI_BIAS_ACT && p.bias && (reinterpret_cast<uintptr_t>(p.bias) & 15) != 0) return false;
-  if (p.epi == TCG_EPI_BIAS_ACT && p.bias && p.bias_period > 1 && ((p.bias_ld % 4) != 0 || p.bias_ld < (p.N + 3) / 4 * 4)) return false;   // 16-byte pieces inside the (padded) table row
+  if (p.epi == TCG_EPI_BIAS_ACT && p.bias && (p.bias_period > 1 || p.rowterm) && ((p.bias_ld % 4) != 0 || p.bias_ld < (p.N + 3) / 4 * 4)) return false;   // 16-byte pieces inside the (padded) table row
+  if (p.rowterm && ((reinterpret_cast<uintptr_t>(p.rowterm) & 15) != 0 || (p.rt_ld % 4) != 0 || p.rt_ld < (p.N + 3) / 4 * 4)) return false;   // ... and the row-group term's
   if (p.epi == TCG_EPI_MASK && p.act && ((reinterpret_cast<uintptr_t>(p.act) & 15) != 0 || (p.ldact % 4) != 0)) return false;
   const int N4 = (p.N + 3) / 4 * 4;                        // 16-byte pieces: a row's last piece may reach into its padding columns
   if (p.ldc < N4 || (p.ldc % 4) != 0 || (reinterpret_cast<uintptr_t>(p.C) & 15) != 0) return false;
@@ -1267,6 +1293,8 @@ int launch_tc_gemm(TcGemmParams p, cudaStream_t s) {
   p.c_vec = ((reinterpret_cast<uintptr_t>(p.C) & 15) == 0 && (p.ldc % 4) == 0) ? 1 : 0;
   p.act_vec = (p.act && (reinterpret_cast<uintptr_t>(p.act) & 15) == 0 && (p.ldact % 4) == 0) ? 1 : 0;
   p.bias_vec = (p.bias && (reinterpret_cast<uintptr_t>(p.bias) & 15) == 0 && (p.bias_ld % 4) == 0) ? 1 : 0;
+  p.rt_vec = (p.rowterm && (reinterpret_cast<uintptr_t>(p.rowterm) & 15) == 0 && (p.rt_ld % 4) == 0) ? 1 : 0;
+  if (p.rowterm && (p.epi != TCG_EPI_BIAS_ACT || !p.bias || p.rt_group < 1)) return fail(GNF_ERR_INVALID, "tensor-core GEMM: a row-group term needs a bias table");
   CUtensorMap tmA, tmB, tmBlo;
   memset(&tmA, 0, sizeof(tmA));
   memset(&tmB, 0, sizeof(tmB));
@@ -1307,17 +1335,19 @@ int launch_tc_gemm(TcGemmParams p, cudaStream_t s) {
                          (2 * kG2Stages + 2 * kG2Ring + 2 * kG2Parts) * sizeof(uint64_t) + 16;
     const int total2 = ((p.M + kGemmBM - 1) / kGemmBM) * ((p.N + kG2BN - 1) / kG2BN);
     const int grid2 = total2 < kNumSMs ? total2 : kNumSMs;
-    cudaFuncSetAttribute(tc_gemm2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2);
-    GNF_LAUNCH_PDL(tc_gemm2_kernel, grid2, kG2Threads, smem2, s, p, tmA, tmB, tmBlo);
+    auto kern2 = p.rowterm ? tc_gemm2_kernel<true> : tc_gemm2_kernel<false>;
+    cudaFuncSetAttribute(kern2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2);
+    GNF_LAUNCH_PDL(kern2, grid2, kG2Threads, smem2, s, p, tmA, tmB, tmBlo);
     return 0;
   }
   p.trace = g_tc_gemm_trace;
   const long long total = (long long)tiles * p.splits;
   const size_t smem = (size_t)stages * stage_bytes + fixed;
   // per launch: the attribute is per DEVICE, a process-wide "done" flag breaks the second GPU of a process (and is racy)
-  cudaFuncSetAttribute(tc_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBudget);
+  auto kern = p.rowterm ? tc_gemm_kernel<true> : tc_gemm_kernel<false>;
+  cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBudget);
   const int grid = (int)(total < kNumSMs ? total : kNumSMs);
-  GNF_LAUNCH_PDL(tc_gemm_kernel, grid, kGemmThreads, smem, s, p, vec_width(p.A, p.lda), vec_width(p.B, p.ldb), tmA, tmB, tmBlo);
+  GNF_LAUNCH_PDL(kern, grid, kGemmThreads, smem, s, p, vec_width(p.A, p.lda), vec_width(p.B, p.ldb), tmA, tmB, tmBlo);
   return 0;
 }
 
@@ -1400,6 +1430,25 @@ int gnf_linear_fwd_tc_ps_tb(const float* X, int ldx, const float* W_hi, const fl
   p.epi = TCG_EPI_BIAS_ACT; p.C = Y; p.ldc = ldy; p.bias = table; p.bias_ld = ldt; p.bias_period = period; p.relu = relu;
   if (int e = launch_tc_gemm(p, (cudaStream_t)stream)) return e;
   return check_launch("gnf_linear_fwd_tc_ps_tb");
+#endif
+}
+
+int gnf_linear_fwd_tc_cond(const float* X, int ldx, const float* W_hi, const float* W_lo, int ldw, const float* table, int ldt, int period,
+                           const float* U, int ldu, int group, float* Y, int ldy, int M, int N, int K, int relu, int passes, gnf_stream_t stream) {
+#ifdef GNF_EMU
+  return gnf::fail(GNF_ERR_UNSUPPORTED, "tensor-core kernels have no host-simulator flavour");
+#else
+  if (!X || !W_hi || !Y || !table || !U || M < 0 || N <= 0 || K <= 0 || ldx < K || ldw < K || ldy < N || ldt < N || ldu < N || period < 1 || group < 1 ||
+      (passes != 1 && passes != 3))
+    return fail(GNF_ERR_INVALID, "gnf_linear_fwd_tc_cond: bad arguments");
+  TcGemmParams p = {};
+  p.A = X; p.lda = ldx; p.a_src = TCG_SRC_K;
+  p.B = W_hi; p.B_lo = W_lo; p.ldb = ldw; p.b_src = TCG_SRC_K;
+  p.M = M; p.N = N; p.K = K; p.passes = passes;
+  p.epi = TCG_EPI_BIAS_ACT; p.C = Y; p.ldc = ldy; p.bias = table; p.bias_ld = ldt; p.bias_period = period; p.relu = relu;
+  p.rowterm = U; p.rt_ld = ldu; p.rt_group = group;
+  if (int e = launch_tc_gemm(p, (cudaStream_t)stream)) return e;
+  return check_launch("gnf_linear_fwd_tc_cond");
 #endif
 }
 

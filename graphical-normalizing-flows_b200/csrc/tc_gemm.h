@@ -24,7 +24,9 @@ struct TcGemmParams {
   const uint32_t* mask_bits; long long mask_ld;         // ... or where bit n of row m is set ([M][mask_ld] words; wins over act)
   uint32_t* bits_out; long long bits_ld;                // TCG_EPI_BIAS_ACT: also emit the bit mask (Y > 0), same layout
   float* rowsum;                                        // engine v2 wgrad only, nullable: rowsum[m] += sum_k A(m, k) (= the bias gradient, atomics)
-  int use_tma, c_vec, act_vec, bias_vec;                          // set by launch_tc_gemm
+  const float* rowterm; long long rt_ld; int rt_group;  // TCG_EPI_BIAS_ACT, nullable: C[m, n] also adds rowterm[(m / rt_group) * rt_ld + n]
+                                                        // (the context term of a conditional DAG flow's layer 1: one row per sample)
+  int use_tma, c_vec, act_vec, bias_vec, rt_vec;                  // set by launch_tc_gemm
   long long* trace;                                     // measurement: SM-clock stamps of CTA 0 (gnf_tc_gemm_set_trace)
 };
 

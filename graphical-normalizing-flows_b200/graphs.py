@@ -35,6 +35,21 @@ def model_graph_state(model):
     return tuple(st)
 
 
+def _static_context(example_context):
+    return example_context.clone() if example_context is not None else None
+
+
+def _load_inputs(static_x, static_ctx, x, context):
+    """Copy a call's inputs into the captured step's static buffers.  A step captured with a context (conditional flows) needs one
+    on every call; one captured without it takes none."""
+    if (static_ctx is None) != (context is None):
+        raise ValueError("this captured step was built " + ("without a context: pass none" if static_ctx is None
+                                                             else "with example_context: pass a context of that shape"))
+    static_x.copy_(x, non_blocking=True)
+    if static_ctx is not None:
+        static_ctx.copy_(context, non_blocking=True)
+
+
 def _capture(body, warmup, stream=None):
     """Warm-up runs and the capture on ONE side stream (`stream`, or a fresh one).  A training loop that keeps capturing new graphs
     (one per quadrature-step count, recaptures after model.step()) should pass the stream it runs its eager steps on: autograd
@@ -56,11 +71,13 @@ def _capture(body, warmup, stream=None):
 class GraphedEvalStep:
     """compute_ll (NormalizingFlow.py:48-50 / UCIExperiments.py:152-162) of a fixed batch shape as one captured graph: the
     evaluation step of the small configs is nine launches of 7-80 us, i.e. launch-bound when issued one by one.
-    Returns (ll [B], z [B,d]) -- static tensors overwritten by the next call."""
+    Returns (ll [B], z [B,d]) -- static tensors overwritten by the next call.  Conditional flows: example_context [B, c] becomes a
+    static buffer as well, and every call passes its context."""
 
-    def __init__(self, model, example_x, warmup=3):
+    def __init__(self, model, example_x, warmup=3, example_context=None):
         self.model, self.warmup = model, warmup
         self.static_x = example_x.clone()
+        self.static_context = _static_context(example_context)
         self.recaptures = 0
         self._capture()
 
@@ -72,16 +89,16 @@ class GraphedEvalStep:
             for cnt in self.counters:
                 ops.counter_add(cnt, 1)
             with torch.no_grad():
-                return model.compute_ll(self.static_x)
+                return model.compute_ll(self.static_x, self.static_context)
 
         self.graph, self.static_out = _capture(body, self.warmup)
         self.state = model_graph_state(model)
 
-    def __call__(self, x):
+    def __call__(self, x, context=None):
         if model_graph_state(self.model) != self.state:      # e.g. model.step() moved an exponent / a gate flag / A
             self.recaptures += 1
             self._capture()
-        self.static_x.copy_(x, non_blocking=True)
+        _load_inputs(self.static_x, self.static_context, x, context)
         self.graph.replay()
         return self.static_out
 
@@ -91,9 +108,10 @@ class GraphedTrainStep:
     exponent, quadrature steps, the addresses of A and of the dual buffers): `model.step()` / `update_dual_param()` /
     `post_process()` may change it, so every call compares `model_graph_state` with the captured one and RECAPTURES when it
     differs (`recaptures` counts them).  Note the reference's own quirk: when update_dual_param re-creates A as a new
-    Parameter, an optimizer built earlier no longer owns it -- here as there."""
+    Parameter, an optimizer built earlier no longer owns it -- here as there.  Conditional flows: example_context [B, c] becomes a
+    static buffer as well, and every call passes its context."""
 
-    def __init__(self, model, optimizer, bucket, example_x, allreduce=True, warmup=3, stream=None, side_branch=True):
+    def __init__(self, model, optimizer, bucket, example_x, allreduce=True, warmup=3, stream=None, side_branch=True, example_context=None):
         self.model, self.opt, self.bucket = model, optimizer, bucket
         has_penalty = any(hasattr(c, "get_power_trace") for c in model.getConditioners())
         self.side = torch.cuda.Stream() if (side_branch and has_penalty and example_x.is_cuda) else None
@@ -102,6 +120,7 @@ class GraphedTrainStep:
             # stream is the default stream
             torch.autograd.graph.set_warn_on_accumulate_grad_stream_mismatch(False)
         self.static_x = example_x.clone()
+        self.static_context = _static_context(example_context)
         self.allreduce, self.warmup, self.stream = allreduce, warmup, stream
         self.recaptures = 0
         self._capture()
@@ -122,11 +141,11 @@ class GraphedTrainStep:
                 self.side.wait_stream(cur)
                 with torch.cuda.stream(self.side):
                     c = model.constraintsLoss()
-                z, jac = model(self.static_x)
+                z, jac = model(self.static_x, self.static_context)
                 cur.wait_stream(self.side)
                 loss = model.loss(z, jac, constraint=c)
             else:
-                z, jac = model(self.static_x)
+                z, jac = model(self.static_x, self.static_context)
                 loss = model.loss(z, jac)
             loss.backward(gradient=self._one)          # a resident cotangent: no ones_like fill launch per step
             if allreduce:
@@ -137,10 +156,10 @@ class GraphedTrainStep:
         self.graph, self.static_loss = _capture(body, self.warmup, self.stream)
         self.state = model_graph_state(model)
 
-    def __call__(self, x):
+    def __call__(self, x, context=None):
         if model_graph_state(self.model) != self.state:
             self.recaptures += 1
             self._capture()
-        self.static_x.copy_(x, non_blocking=True)
+        _load_inputs(self.static_x, self.static_context, x, context)
         self.graph.replay()
         return self.static_loss

@@ -67,7 +67,8 @@ def _note_flops(name, flops, shape=None):
 
 def tc_kernel_name(op, M, N, K, passes=3):
     """Which kernel of the tcgen05 GEMM engine a layer call of this shape launches (mirrors g2_eligible / w2_eligible in
-    csrc/tc_gemm.cu for TMA-loadable operands): op 'fwd' / 'dgrad' (M rows, N out-features, K in-features) or 'wgrad'."""
+    csrc/tc_gemm.cu for TMA-loadable operands, and for bias tables / context terms with rows of 16-byte pieces, as DagMlpFn
+    makes them): op 'fwd' / 'dgrad' (M rows, N out-features, K in-features) or 'wgrad'."""
     if passes == 3:
         if op == "wgrad":
             return "tc_wgrad2_kernel" if (N >= 256 and (K >= 256 or 32 <= K <= 64) and M >= 2048) else "tc_gemm_kernel"
@@ -734,22 +735,45 @@ def _dag_l1_plane(M, N1, d):
     return DAG_L1_PLANE and d >= DAG_L1_PLANE_MIN_D and M > 0 and _gemm_passes(M, N1, d) != 0 and not L._SIMULATOR
 
 
+def _dag_context_term(context, W1, in_net, N1):
+    """U = context W1[:, in_net:]^T ([B, N1], rows padded to 16-byte pieces): the per-sample term of a conditional flow's layer 1."""
+    B, c = context.shape
+    U = _rows(B, N1, context)
+    if B > 0:
+        _call("gnf_linear_fwd", ptr(context), c, ptr(W1[:, in_net:]), W1.stride(0), None, 1, ptr(U), U.stride(0), B, N1, c, 0, stream_ptr())
+        _count()
+    return U
+
+
 class DagMlpFn(torch.autograd.Function):
     """DAGConditioner.forward (DAGConditioner.py:126-169): gate/threshold of A, masked expansion of x,
     optional one-hot encoding, embedding MLP — with the [B,d,d] masked tensor generated inside the first
-    GEMM's operand loader.  forward(x, A, gate, hot, *params) -> h [B, d, H]."""
+    GEMM's operand loader.  forward(x, A, gate, hot, *params) -> h [B, d, H], params = W0, b0, W1, b1, ...
+
+    Conditional flows: params may end with a context [B, c] after the last bias (an odd count).  Layer 1 then has in_net + c
+    inputs, in_net = 2 d (hot) or d, and its input row for sample b, variable i is [e[b,i,:] | onehot(i) | context[b,:]]:
+    y1[b*d+i] = act(e[b,i,:] W1[:, :d]^T + T[i] + U[b]) with the bias table T (one-hot columns + b1) and
+    U = context W1[:, in_net:]^T, added in the epilogue of whichever layer-1 kernel runs."""
 
     @staticmethod
     def forward(ctx, x, A, gate, hot, *params):
         require(x, "x")
         A = require(_contig(A), "A")
+        context = None
+        if len(params) % 2:
+            params, context = params[:-1], require(params[-1], "context")
         weights = [require(_contig(p), "weight") for p in params[0::2]]
         biases = [require(_contig(p), "bias") for p in params[1::2]]
         B, d = x.shape
         n = len(weights)
         _SPLIT_CACHE.clear()     # weight splits live from a forward to its own backward only
-        if weights[0].shape[1] != (2 * d if hot else d):
-            raise ValueError(f"DAGConditioner: first layer expects {weights[0].shape[1]} inputs, d={d}, hot_encoding={hot}")
+        in_net = 2 * d if hot else d
+        c = weights[0].shape[1] - in_net
+        if c < 0 or (c > 0) != (context is not None):
+            raise ValueError(f"DAGConditioner: first layer expects {weights[0].shape[1]} inputs, d={d}, hot_encoding={hot}, "
+                             f"context={'none' if context is None else tuple(context.shape)}")
+        if context is not None and tuple(context.shape) != (B, c):
+            raise ValueError(f"DAGConditioner: context must be [B, cond_in] = [{B}, {c}], got {tuple(context.shape)}")
         for t in (gate.noise or ()):
             require(t, "noise")
             if tuple(t.shape) != (B, d, d):
@@ -764,7 +788,13 @@ class DagMlpFn(torch.autograd.Function):
         tc_fwd = (DAG_L1_NARROW_TC_FWD and DAG_L1_KEEP_GATES and d <= 64 and gate.mode != L.GATE_TABLE and B > 0 and n > 1 and hot
                   and DAG_L1_NARROW_TC and _GEMM_MODE in ("auto", "tf32x3", "auto-fast", "tf32") and not L._SIMULATOR
                   and B * d >= 2048 and N1 >= 256 and d >= 32)        # evaluation (no gradient) takes it as well
-        if tc_fwd:
+        U = None
+        if context is not None:
+            # conditional: the table keeps rows of 16-byte pieces on every route (engine v2 reads it so, period 1 included)
+            T = torch.empty(d if hot else 1, _pad4(N1), device=x.device, dtype=x.dtype)
+            _call("gnf_dag_bias_table_ld", ptr(weights[0]), weights[0].stride(0), ptr(biases[0]), ptr(T), T.stride(0), d, N1, int(hot), st)
+            U = _dag_context_term(context, weights[0], in_net, N1)
+        elif tc_fwd:
             T = torch.empty(d, _pad4(N1), device=x.device, dtype=x.dtype)
             _call("gnf_dag_bias_table_ld", ptr(weights[0]), weights[0].stride(0), ptr(biases[0]), ptr(T), T.stride(0), d, N1, 1, st)
         else:
@@ -788,7 +818,19 @@ class DagMlpFn(torch.autograd.Function):
                 gate_planes = (_rows(B * d, d, x), _rows(B * d, d, x))        # de/dx, de/dP (same row stride as E): the backward reduction streams them
             _call("gnf_dag_embed_fwd", ptr(x), ptr(P), C.byref(g), ptr(E), ptr(gate_planes[0]), ptr(gate_planes[1]), E.stride(0), B, d, st)
             W1e = weights[0][:, :d]                 # the masked-input half of layer 1; the one-hot half is the bias table T
-            linear_fwd(E, W1e, T, relu=(n > 1), bias_period=(d if hot else 1), out=y, ldy=y.stride(0), K=d, ldx=E.stride(0))
+            if U is not None:
+                passes = _gemm_passes(B * d, N1, d)
+                if passes == 3 and _tma_ok(E, E.stride(0)):
+                    hi, lo = _split_weight(W1e)
+                else:
+                    hi, lo = _tma_weight(W1e), None
+                _note_flops("gnf_linear_fwd_tc", 2. * B * d * N1 * d, (B * d, N1, d))
+                _TIMES_ALIAS["gnf_linear_fwd_tc_cond"] = "gnf_linear_fwd_tc"
+                _call("gnf_linear_fwd_tc_cond", ptr(E), E.stride(0), ptr(hi), ptr(lo), hi.stride(0), ptr(T), T.stride(0), (d if hot else 1),
+                      ptr(U), U.stride(0), d, ptr(y), y.stride(0), B * d, N1, d, int(n > 1), passes, st)
+                _count()
+            else:
+                linear_fwd(E, W1e, T, relu=(n > 1), bias_period=(d if hot else 1), out=y, ldy=y.stride(0), K=d, ldx=E.stride(0))
             _count(2)
         elif (DAG_L1_KEEP_GATES and d <= 64 and gate.mode != L.GATE_TABLE and B > 0 and (any(ctx.needs_input_grad) or tc_fwd)):
             # narrow flow, stochastic gate, training: the forward leaves e, de/dx, de/dP ([B d, 64] each) for the two backward kernels
@@ -797,15 +839,30 @@ class DagMlpFn(torch.autograd.Function):
                 _TIMES_ALIAS["gnf_dag_gate_planes"] = "gnf_dag_l1_fwd"
                 _call("gnf_dag_gate_planes", ptr(x), ptr(P), C.byref(g), ptr(narrow[0]), ptr(narrow[1]), ptr(narrow[2]), B, d, st)
                 hi, lo = _split_weight(weights[0][:, :d])
-                _TIMES_ALIAS["gnf_linear_fwd_tc_ps_tb"] = "gnf_dag_l1_fwd"
-                _call("gnf_linear_fwd_tc_ps_tb", ptr(narrow[0]), 64, ptr(hi), ptr(lo), hi.stride(0), ptr(T), T.stride(0), d, ptr(y), y.stride(0),
-                      B * d, N1, d, 1, st)
+                if U is not None:
+                    _TIMES_ALIAS["gnf_linear_fwd_tc_cond"] = "gnf_dag_l1_fwd"
+                    _call("gnf_linear_fwd_tc_cond", ptr(narrow[0]), 64, ptr(hi), ptr(lo), hi.stride(0), ptr(T), T.stride(0), d, ptr(U), U.stride(0), d,
+                          ptr(y), y.stride(0), B * d, N1, d, 1, 3, st)
+                else:
+                    _TIMES_ALIAS["gnf_linear_fwd_tc_ps_tb"] = "gnf_dag_l1_fwd"
+                    _call("gnf_linear_fwd_tc_ps_tb", ptr(narrow[0]), 64, ptr(hi), ptr(lo), hi.stride(0), ptr(T), T.stride(0), d, ptr(y), y.stride(0),
+                          B * d, N1, d, 1, st)
                 _count(4)
+            elif U is not None:
+                _TIMES_ALIAS["gnf_dag_l1_fwd_cond"] = "gnf_dag_l1_fwd"
+                _call("gnf_dag_l1_fwd_cond", ptr(x), ptr(P), C.byref(g), ptr(weights[0]), weights[0].stride(0), ptr(T), T.stride(0), (d if hot else 1),
+                      ptr(U), U.stride(0), ptr(y), y.stride(0), ptr(narrow[0]), ptr(narrow[1]), ptr(narrow[2]), B, d, N1, int(n > 1), st)
+                _count(3)
             else:
                 _TIMES_ALIAS["gnf_dag_l1_fwd_save"] = "gnf_dag_l1_fwd"
                 _call("gnf_dag_l1_fwd_save", ptr(x), ptr(P), C.byref(g), ptr(weights[0]), weights[0].stride(0), ptr(T), (d if hot else 1),
                       ptr(y), y.stride(0), ptr(narrow[0]), ptr(narrow[1]), ptr(narrow[2]), B, d, N1, int(n > 1), st)
                 _count(3)
+        elif U is not None:
+            _TIMES_ALIAS["gnf_dag_l1_fwd_cond"] = "gnf_dag_l1_fwd"
+            _call("gnf_dag_l1_fwd_cond", ptr(x), ptr(P), C.byref(g), ptr(weights[0]), weights[0].stride(0), ptr(T), T.stride(0), (d if hot else 1),
+                  ptr(U), U.stride(0), ptr(y), y.stride(0), None, None, None, B, d, N1, int(n > 1), st)
+            _count(3)
         else:
             _call("gnf_dag_l1_fwd", ptr(x), ptr(P), C.byref(g), ptr(weights[0]), weights[0].stride(0), ptr(T), (d if hot else 1),
                                        ptr(y), y.stride(0), B, d, N1, int(n > 1), st)
@@ -825,6 +882,7 @@ class DagMlpFn(torch.autograd.Function):
         ctx.narrow = narrow if any(ctx.needs_input_grad) else None
         ctx.save_for_backward(x, A, P, dPdA, *weights, *acts)
         ctx.gate, ctx.hot, ctx.n = gate, hot, n
+        ctx.context, ctx.in_net = context, in_net
         if n == 1:
             cur = cur.view(B, d, -1).clone()
         return cur
@@ -865,8 +923,27 @@ class DagMlpFn(torch.autograd.Function):
                 _call("gnf_dag_l1_wgrad_saved", ptr(delta), delta.stride(0), ptr(narrow[0]), ptr(dW1), W1.stride(0), B, d, N1, st)
             else:
                 _call("gnf_dag_l1_wgrad", ptr(delta), delta.stride(0), ptr(x), ptr(P), C.byref(g), ptr(dW1), W1.stride(0), B, d, N1, st)
+        context, in_net = ctx.context, ctx.in_net
+        ctx.context = None
+        dctx = None
         with _Fork(1, x) as f_b:
-            dT = colsum(delta, delta.stride(0), M, N1, period=(d if hot else 1))
+            if context is None:
+                dT = colsum(delta, delta.stride(0), M, N1, period=(d if hot else 1))
+            else:
+                # conditional: the table's gradient and the per-sample sums S[b] = sum_i delta[b*d+i] from one read of delta, then
+                # dW1[:, in_net:] = S^T context and dcontext = S W1[:, in_net:] (FFMA engine: B x N1 x c, strict fp32 in every mode)
+                c = context.shape[1]
+                dT = torch.empty(d if hot else 1, N1, device=x.device, dtype=x.dtype)
+                S = _rows(B, N1, x)
+                stb = stream_ptr()
+                _call("gnf_dag_l1_bias_sums", ptr(delta), delta.stride(0), ptr(dT), ptr(S), S.stride(0), B, d, N1, (d if hot else 1), stb)
+                _call("gnf_linear_wgrad", ptr(S), S.stride(0), ptr(context), c, ptr(dW1[:, in_net:]), dW1.stride(0), B, N1, c, stb)
+                _count(2)
+                if needs[4 + 2 * n]:
+                    dctx = torch.empty_like(context)
+                    if B > 0:
+                        _call("gnf_linear_dgrad", ptr(S), S.stride(0), ptr(W1[:, in_net:]), W1.stride(0), None, 0, ptr(dctx), c, B, N1, c, stb)
+                        _count()
             db1 = torch.empty(N1, device=x.device, dtype=x.dtype)
             _call("gnf_dag_bias_table_bwd", ptr(dT), ptr(dW1), W1.stride(0), ptr(db1), d, N1, int(hot), stream_ptr())
         _count(2)
@@ -905,6 +982,8 @@ class DagMlpFn(torch.autograd.Function):
         out = [dx if needs[0] else None, dA if needs[1] else None, None, None]
         for l in range(n):
             out += [dWs[l], dbs[l]]
+        if context is not None:
+            out.append(dctx)
         return tuple(out)
 
 

@@ -152,6 +152,16 @@ int gnf_linear_fwd_tc_ps_tb(const float* X, int ldx, const float* W_hi, const fl
                             int period, float* Y, int ldy, int M, int N, int K, int relu, gnf_stream_t stream);
 int gnf_linear_dgrad_tc_ps(const float* dY, int lddy, const float* W_hi, const float* W_lo, int ldw, const float* act, int ldact,
                            float* dX, int lddx, int M, int N, int K, gnf_stream_t stream);
+/* Layer 1 of a conditional DAG flow (DAGConditioner with cond_in = c > 0) on the tensor-core engine, against the embedding plane X:
+ *   Y[m, n] = act( sum_k X[m, k] W[n, k] + table[m % period, n] + U[m / group, n] ),
+ * U = context W1[:, in_net:]^T ([B, N] with row stride ldu, group = d: one row per sample).  The reference builds layer 1 with
+ * in_net + cond_in inputs (DAGMLP, DAGConditioner.py:7-20) and never feeds the context in (its forward, :126-169, quirk Q8); the
+ * column order [e | one-hot | context] of that layout defines the term.  passes 3: W_hi / W_lo as for gnf_linear_fwd_tc_ps, or
+ * W_lo = NULL with W_hi = W (split per tile); passes 1: single-pass TF32, W_hi = W, W_lo ignored.  table [period, ldt] and U in
+ * 16-byte pieces (16-byte aligned, ldt and ldu multiples of 4 floats, >= round_up(N, 4)) are what engine v2 takes. */
+int gnf_linear_fwd_tc_cond(const float* X, int ldx, const float* W_hi, const float* W_lo, int ldw, const float* table, int ldt,
+                           int period, const float* U, int ldu, int group, float* Y, int ldy, int M, int N, int K, int relu, int passes,
+                           gnf_stream_t stream);
 /* Host-only query of that plan for a GEMM of M x N outputs reduced over K (wgrad != 0: the split-K orientation, where M x N is
  * the weight shape and K the number of rows): writes the tile width and the split-K factor the engine would use. */
 int gnf_tc_gemm_plan(int M, int N, int K, int passes, int wgrad, int* bn, int* splits);
@@ -221,6 +231,19 @@ int gnf_dag_l1_dgrad(const float* dY, int lddy, const float* W1, int ldw, const 
 int gnf_dag_l1_fwd_save(const float* x, const float* P, const gnf_gate_t* gate, const float* W1, int ldw, const float* T,
                         int bias_period, float* Y, int ldy, float* E, float* DX, float* DP, int B, int d, int N, int relu,
                         gnf_stream_t stream);
+/* Conditional DAG flows (cond_in = c > 0): layer 1's input row for sample b, variable i is [e[b,i,:] | onehot(i) | context[b,:]]
+ * (the in_net + cond_in columns of DAGMLP's first Linear, DAGConditioner.py:7-20), so
+ *   Y[b*d+i, n] = act( sum_j e[b,i,j] W1[n,j] + T[i or 0, n] + U[b, n] ),   U = context W1[:, in_net:]^T  ([B, N], row stride ldu).
+ * The FFMA flavours of gnf_dag_l1_fwd (E = DX = DP = NULL) and gnf_dag_l1_fwd_save (all three planes, d <= 64) with the context
+ * term; T has row stride ldt.  bias_period: d (hot encoding) or 1. */
+int gnf_dag_l1_fwd_cond(const float* x, const float* P, const gnf_gate_t* gate, const float* W1, int ldw, const float* T, int ldt,
+                        int bias_period, const float* U, int ldu, float* Y, int ldy, float* E, float* DX, float* DP, int B, int d, int N,
+                        int relu, gnf_stream_t stream);
+/* Backward of the two bias terms of that layer from one read of its pre-activation cotangent delta ([B*d, N], row stride ldd):
+ *   dT[i % period, n] = sum_b delta[b*d+i, n]   (the bias table's gradient, = gnf_colsum with that period; period d or 1)
+ *   S[b, n]           = sum_i delta[b*d+i, n]   (per sample, row stride lds: dW1[:, in_net:] = S^T context, dcontext = S W1[:, in_net:]).
+ * Both are overwritten. */
+int gnf_dag_l1_bias_sums(const float* delta, int ldd, float* dT, float* S, int lds, int B, int d, int N, int period, gnf_stream_t stream);
 /* ... the three planes alone (layer 1's forward then is gnf_linear_fwd_tc_ps against E with the bias table as a periodic bias). */
 int gnf_dag_gate_planes(const float* x, const float* P, const gnf_gate_t* gate, float* E, float* DX, float* DP, int B, int d,
                         gnf_stream_t stream);
