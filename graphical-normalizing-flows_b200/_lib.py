@@ -107,6 +107,7 @@ _PROTOS = {
     "gnf_umnn_saved_floats_per_node_row": ([C.POINTER(MlpT)], _SZ),
     "gnf_umnn_fwd": ([_P, _P, C.POINTER(MlpT), _I, _P, _P, _P, _P, _P, _P, _P, _I, _I, _P, _SZ, _P], C.c_int),
     "gnf_umnn_invert": ([_P, _P, C.POINTER(MlpT), _I, _P, _P, _P, _I, _F, _F, _I, _P, _SZ, _P], C.c_int),
+    "gnf_umnn_bwd_workspace_bytes": ([C.POINTER(MlpT)], _SZ),
     "gnf_umnn_bwd": ([_P, _P, C.POINTER(MlpT), _I, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, C.POINTER(MlpGradT), _I, _I,
                       _P, _SZ, _P], C.c_int),
     "gnf_umnn_tc_workspace_bytes": ([C.POINTER(MlpT)], _SZ),

@@ -680,6 +680,12 @@ __global__ void __launch_bounds__(kUThreads) umnn_bwd_kernel(UmnnBwdParams p) {
 
 static size_t fwd_smem_bytes(int NP) { return fwd_smem_bytes_for(NP); }
 static size_t bwd_smem_bytes(int NP, int KP0, int L) { return ((size_t)KP0 * kLDR + (size_t)L * NP * kLDR + 2 * kKC * NP + 256 + 128) * sizeof(float); }
+// The backward keeps every hidden layer's tile in shared memory: deep or wide integrands (e.g. [256, 256, 256]) do not fit.
+static int bwd_smem_check(int NP, int KB0, int L) {
+  const size_t smem = bwd_smem_bytes(NP, KB0, L);
+  if (smem > 227 * 1024) return fail(GNF_ERR_UNSUPPORTED, "umnn bwd: %d hidden layers of padded width %d need %zu B of shared memory (> 227 KB)", L, NP, smem);
+  return 0;
+}
 
 template <int TN>
 static int launch_fwd(const UmnnFwdParams& p, cudaStream_t s) {
@@ -697,8 +703,8 @@ static int launch_fwd(const UmnnFwdParams& p, cudaStream_t s) {
 }
 template <int TN>
 static int launch_bwd(const UmnnBwdParams& p, cudaStream_t s) {
+  if (int e = bwd_smem_check(16 * TN, p.pk.kb0, p.pk.L)) return e;
   const size_t smem = bwd_smem_bytes(16 * TN, p.pk.kb0, p.pk.L);
-  if (smem > 227 * 1024) return fail(GNF_ERR_UNSUPPORTED, "umnn bwd: %d hidden layers of padded width %d need %zu B of shared memory (> 227 KB)", p.pk.L, 16 * TN, smem);
 #ifndef GNF_EMU
   cudaFuncSetAttribute(umnn_bwd_kernel<TN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
 #endif
@@ -719,6 +725,14 @@ size_t gnf_umnn_workspace_bytes(const gnf_mlp_t* net) {
   PackPlan pl;
   int TN;
   if (make_plan(net, &pl, &TN)) return 0;
+  return pl.total * sizeof(float);
+}
+
+size_t gnf_umnn_bwd_workspace_bytes(const gnf_mlp_t* net) {
+  PackPlan pl;
+  int TN;
+  if (make_plan(net, &pl, &TN)) return 0;
+  if (bwd_smem_check(pl.NP, pl.KB0, net->n_layers - 1)) return 0;
   return pl.total * sizeof(float);
 }
 

@@ -1027,11 +1027,32 @@ def _umnn_tc3_takes(net, R, S):
     return UMNN_FWD_FUSED_TC3 and S + 1 <= UMNN_TC3_MAX_NODES and lib().gnf_umnn_tc3_workspace_bytes(C.byref(net), R) != 0
 
 
+_UMNN_LW_PASSES = {"ffma": 0, "tf32": 1, "tf32x3": 3, "auto": 3, "auto-fast": 3}
+
+
+def _umnn_fused_ffma_fallback(net, R, S, train, fast, device):
+    """Route of a call that the choice above left on the fused FFMA kernels: None when they take the integrand (the forward and,
+    in training, the backward, whose shared-memory tiles of every hidden layer cap depth x width); otherwise the layer-wise
+    passes of the GEMM mode.  Raises, before any work is done, when no engine takes the call."""
+    ffma_fwd = fast or lib().gnf_umnn_workspace_bytes(C.byref(net)) != 0
+    if ffma_fwd and (not train or lib().gnf_umnn_bwd_workspace_bytes(C.byref(net)) != 0):
+        return None
+    why = lib().gnf_last_error().decode()
+    if not fast and UMNN_ENGINE == "auto" and net.dims[0] >= 2:
+        need = 4 * (lib().gnf_umnn_lw_saved_floats(C.byref(net), R, S, int(train)) +
+                    (lib().gnf_umnn_lw_workspace_bytes(C.byref(net), R, S, int(train)) // 4))
+        if 0 < need <= _activation_budget(device):
+            return _UMNN_LW_PASSES[_GEMM_MODE]
+        why += "; layer-wise engine: " + (lib().gnf_last_error().decode() if need == 0 else
+                                          f"{need} B of activations exceed the budget (ops.SAVE_ACTIVATIONS_MAX_BYTES)")
+    raise RuntimeError("libgnf: " + why)
+
+
 def _umnn_layerwise_passes(net, R, S, train, device=None):
     """GEMM passes (0 FFMA / 1 TF32 / 3 3xTF32) for the layer-wise UMNN engine, or None for the fused FFMA kernels."""
     if UMNN_ENGINE == "fused" or net.dims[0] < 2:
         return None
-    passes = {"ffma": 0, "tf32": 1, "tf32x3": 3, "auto": 3, "auto-fast": 3}[_GEMM_MODE]
+    passes = _UMNN_LW_PASSES[_GEMM_MODE]
     if UMNN_ENGINE == "auto":
         hidden = [net.dims[l] for l in range(1, net.n_layers)]
         if passes == 0 or net.n_layers < 3 or min(hidden) < 64 or R * (S + 2) < UMNN_LAYERWISE_MIN_NODE_ROWS:
@@ -1097,10 +1118,18 @@ class UmnnFn(torch.autograd.Function):
             raise ValueError(f"integrand expects {weights[0].shape[1] - 1} conditioning features, h has {E}")
         R = B * d
         net = _mlp_struct(weights, biases)
-        nbytes = (lib().gnf_umnn_tc_workspace_bytes if fast else lib().gnf_umnn_workspace_bytes)(C.byref(net))
-        if nbytes == 0:
-            raise RuntimeError("libgnf: " + lib().gnf_last_error().decode())
-        ws = torch.empty((nbytes + 3) // 4, device=x.device, dtype=torch.float32)
+        if fast:
+            nbytes = lib().gnf_umnn_tc_workspace_bytes(C.byref(net))
+            if nbytes == 0:
+                raise RuntimeError("libgnf: " + lib().gnf_last_error().decode())
+        train = any(ctx.needs_input_grad)
+        lw_passes = None if fast else _umnn_layerwise_passes(net, R, int(S), train, x.device)
+        if lw_passes is None:
+            lw_passes = _umnn_fused_ffma_fallback(net, R, int(S), train, fast, x.device)
+        if lw_passes is None:
+            if not fast:
+                nbytes = lib().gnf_umnn_workspace_bytes(C.byref(net))
+            ws = torch.empty((nbytes + 3) // 4, device=x.device, dtype=torch.float32)
         ccw, ccn = cc_weights(S, x.device)
         z = torch.empty_like(x)
         jac = torch.empty_like(x)
@@ -1108,8 +1137,6 @@ class UmnnFn(torch.autograd.Function):
         logdet = torch.empty(B, device=x.device, dtype=x.dtype)
         saved = None
         tc3 = False
-        train = any(ctx.needs_input_grad)
-        lw_passes = None if fast else _umnn_layerwise_passes(net, R, int(S), train, x.device)
         if fast:
             _call("gnf_umnn_fwd_tc", ptr(x), ptr(h), C.byref(net), int(S), ptr(ccw), ptr(ccn), ptr(z), ptr(zrev), ptr(jac),
                   ptr(logdet), R, d, ptr(ws), nbytes, stream_ptr())
@@ -1168,8 +1195,6 @@ class UmnnFn(torch.autograd.Function):
         B, d = x.shape
         R = B * d
         net = _mlp_struct(weights, biases)
-        nbytes = lib().gnf_umnn_workspace_bytes(C.byref(net))
-        ws = torch.empty((nbytes + 3) // 4, device=x.device, dtype=torch.float32)
         ccw, ccn = cc_weights(ctx.S, x.device)
         gz = _contig(gz) if gz is not None else None
         gjac = _contig(gjac) if gjac is not None else None
@@ -1200,6 +1225,8 @@ class UmnnFn(torch.autograd.Function):
                   nbytes, stream_ptr())
             _count(4 + 3 * n)
         else:
+            nbytes = lib().gnf_umnn_bwd_workspace_bytes(C.byref(net))
+            ws = torch.empty((nbytes + 3) // 4, device=x.device, dtype=torch.float32)
             _call("gnf_umnn_bwd", ptr(x), ptr(h), C.byref(net), ctx.S, ptr(ccw), ptr(ccn), ptr(jac), ptr(gz), ptr(gzrev), ptr(gjac),
                   ptr(glogdet), ptr(ctx.saved_acts), ptr(dx), ptr(dh), C.byref(grads), R, d, ptr(ws), nbytes, stream_ptr())
         ctx.saved_acts = None

@@ -308,7 +308,10 @@ int gnf_umnn_invert(const float* z, const float* h, const gnf_mlp_t* net, int S,
                     int iters, float lo, float hi, int R, void* work, size_t work_bytes, gnf_stream_t stream);
 /* Cotangents: gz [R], gzrev [R], gjac [R], glogdet [R/d], each nullable (NULL = zero cotangent).
  * Gradient convention = UMNN's: dtheta, dh by quadrature of the integrand's gradients with weights
- * w_k*gz*x/2; dx by the Leibniz rule f(x)*gz; the jac output is differentiated by the plain chain rule. */
+ * w_k*gz*x/2; dx by the Leibniz rule f(x)*gz; the jac output is differentiated by the plain chain rule.
+ * work: gnf_umnn_bwd_workspace_bytes(net) bytes.  Host-only query: 0 when gnf_umnn_bwd refuses the integrand (see
+ * gnf_last_error), i.e. when its forward does or when the tiles of every hidden layer exceed 227 KB of shared memory. */
+size_t gnf_umnn_bwd_workspace_bytes(const gnf_mlp_t* net);
 int gnf_umnn_bwd(const float* x, const float* h, const gnf_mlp_t* net, int S, const float* ccw, const float* ccn,
                  const float* jac, const float* gz, const float* gzrev, const float* gjac, const float* glogdet,
                  const float* saved, float* dx, float* dh, const gnf_mlp_grad_t* grads, int R, int d, void* work,

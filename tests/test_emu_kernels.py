@@ -42,6 +42,58 @@ def test_golden_monotonic_case_layerwise_engine_in_simulator(emu, name):
         G.ops.UMNN_ENGINE = "auto"
 
 
+def _record_calls(monkeypatch):
+    """Names of the C-ABI entry points UmnnFn calls (kernel timing has no simulator flavour)."""
+    calls = []
+    real = G.ops._call
+
+    def rec(name, *args):
+        calls.append(name)
+        return real(name, *args)
+    monkeypatch.setattr(G.ops, "_call", rec)
+    return calls
+
+
+def test_training_on_a_net_the_ffma_backward_refuses_runs_layerwise_in_simulator(emu, monkeypatch):
+    """[256, 256, 256] under the default engine and GEMM mode 'ffma': the FFMA backward cannot hold its tiles in shared memory, so
+    the training step runs gnf_umnn_fwd_lw + gnf_umnn_bwd_lw with FFMA GEMMs, against float64."""
+    from umnn_ref import OUTS, explicit_quadrature, grad_names, make_cots, make_params, rel
+    torch.set_num_threads(1)
+    assert G.ops.UMNN_ENGINE == "auto" and G.ops.get_gemm_mode() == "ffma"
+    B, d, E, S = 1, 2, 3, 3
+    params = [p.requires_grad_(True) for p in make_params([256, 256, 256], E, 0, "cpu")]
+    g = torch.Generator().manual_seed(1)
+    x, h = torch.randn(B, d, generator=g).requires_grad_(True), torch.randn(B, d, E, generator=g).requires_grad_(True)
+    cots = make_cots(OUTS, B, d, "cpu", 2)
+    calls = _record_calls(monkeypatch)
+    outs = G.ops.UmnnFn.apply(x, h, S, True, False, *params)
+    grads = torch.autograd.grad(outs, [x, h] + params, [cots[k] for k in OUTS])
+    assert {c for c in calls if c.startswith("gnf_umnn")} == {"gnf_umnn_fwd_lw", "gnf_umnn_bwd_lw"}, calls
+    ref = explicit_quadrature(params, x, h, S, cots)
+    got = dict(zip(OUTS + tuple(grad_names(4)), [o.detach() for o in outs] + list(grads)))
+    errs = {k: rel(got[k], ref[k], k, d) for k in ref}
+    bad = {k: e for k, e in errs.items() if not e < (1e-6 if k in OUTS else 2e-4)}
+    assert not bad, bad
+
+
+def test_no_umnn_engine_for_the_call_raises_before_any_work_in_simulator(emu, monkeypatch):
+    """Training [256, 256, 256] with the engine forced to 'fused', or with no activation budget for the layer-wise engine: UmnnFn
+    raises in its forward, before any entry point runs."""
+    from umnn_ref import make_params
+    params = [p.requires_grad_(True) for p in make_params([256, 256, 256], 3, 0, "cpu")]
+    x, h = torch.randn(1, 2, requires_grad=True), torch.randn(1, 2, 3, requires_grad=True)
+    calls = _record_calls(monkeypatch)
+    for name, value in [("UMNN_ENGINE", "fused"), ("SAVE_ACTIVATIONS_MAX_BYTES", 0)]:
+        old = getattr(G.ops, name)
+        setattr(G.ops, name, value)
+        try:
+            with pytest.raises(RuntimeError, match="shared memory"):
+                G.ops.UmnnFn.apply(x, h, 3, True, False, *params)
+        finally:
+            setattr(G.ops, name, old)
+    assert not calls, calls
+
+
 def test_power_trace_golden_in_simulator(emu):
     """K2 against the reference's golden power traces, both flavours: the no-grad forward (torch.matrix_power's order) and
     the training forward that leaves (I + alpha A∘A)^(p-1) for an elementwise backward (d <= 64)."""

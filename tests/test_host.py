@@ -232,6 +232,43 @@ def test_fused_umnn_backward_takes_every_net_the_fused_forward_takes():
     assert accepted == 10 ** 2 + 10 ** 3
 
 
+def test_ffma_umnn_backward_query_matches_its_shared_memory_limit():
+    """gnf_umnn_bwd_workspace_bytes is non-zero exactly when gnf_umnn_bwd takes the integrand: the forward's plan (1 + E padded
+    to 16 within the padded hidden width 16 TN) and the backward's tiles, (KB0 68 + L NP 68 + 32 NP + 384) floats <= 227 KB,
+    over 2..8 linear layers, the largest hidden width on both sides of every TN step, and E at 1, 31, 32, 223, 255.
+    Host-only query (the weight pointers are never read)."""
+    import ctypes as C
+    import __graft_entry__
+    __graft_entry__.build()
+    lib = G._lib.load_library()
+    widths = (1, 16, 32, 33, 64, 65, 112, 113, 160, 161, 208, 209, 255, 256)
+    seen = set()
+    for n_layers in range(2, 9):
+        for w in widths:
+            for hidden in {(w,) * (n_layers - 1), (1,) * (n_layers - 2) + (w,)}:
+                for E in (1, 31, 32, 223, 255):
+                    TN = next(t for t in (2, 4, 7, 10, 13, 16) if 16 * t >= w)
+                    NP, KP0, KB0 = 16 * TN, -(-(1 + E) // 16) * 16, -(-(1 + E) // 32) * 32
+                    fits = KP0 <= NP and (KB0 * 68 + len(hidden) * NP * 68 + 32 * NP + 384) * 4 <= 227 * 1024
+                    net = G._lib.MlpT()
+                    dims = [1 + E, *hidden, 1]
+                    net.n_layers = len(dims) - 1
+                    for i, v in enumerate(dims):
+                        net.dims[i] = v
+                    got = lib.gnf_umnn_bwd_workspace_bytes(C.byref(net))
+                    assert (got != 0) == fits, (hidden, E, got, lib.gnf_last_error())
+                    if fits:
+                        assert got == lib.gnf_umnn_workspace_bytes(C.byref(net))
+                    seen.add(fits)
+    assert seen == {True, False}
+    net = G._lib.MlpT()
+    for i, v in enumerate([8, 256, 256, 256, 1]):
+        net.dims[i] = v
+    net.n_layers = 4
+    assert lib.gnf_umnn_workspace_bytes(C.byref(net)) > 0 and lib.gnf_umnn_bwd_workspace_bytes(C.byref(net)) == 0
+    assert b"shared memory" in lib.gnf_last_error()
+
+
 # ---------------- experiment plumbing (SURVEY 8f rank 4) ----------------
 def test_reference_yaml_preset_and_driver_defaults(tmp_path):
     """A preset in the reference's YAML format (UCIExperimentsConfigurations.yml:1-14) merged over the driver's argparse defaults;
