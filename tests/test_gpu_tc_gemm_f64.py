@@ -38,36 +38,18 @@ import pytest
 import torch
 
 import gnf_b200 as G
+from gemm_ref import NAN, SENT, Mat, assert_engines, check_sentinels, cw_err, launched, pad4, poison  # noqa: F401 (poison: fixture)
 
-SENT = -777.0                      # outputs: every element the kernel must not write
 GARBAGE = 1234.5                   # padding columns of a bias table: finite, so a read shows up as a wrong value
-NAN = float("nan")                 # operand padding: a read shows up as NaN
 V1, V2, W2, CS, SPLIT = "tc_gemm_kernel", "tc_gemm2_kernel", "tc_wgrad2_kernel", "colsum_kernel", "split_tf32_kernel"
 ENGINES = (V1, V2, W2, CS, SPLIT)
 FLOOR = {"fwd": 8e-7, "dgrad": 8e-7, "wgrad": 8e-7, "db": 1e-7}
 TF32_BAR = 2e-3
 
 
-def pad4(n):
-    return (n + 3) // 4 * 4
-
-
 # ---------------------------------------------------------------------------------------------------------------------
-# harness
+# harness (Mat, sentinels, launched kernels, the componentwise metric, the poison fixture: gemm_ref.py)
 # ---------------------------------------------------------------------------------------------------------------------
-@pytest.fixture
-def poison():
-    """Returns a function that NaN-fills free blocks in the small (<= 1 MB) and the large pool of the caching allocator and
-    releases them again (no empty_cache): the next torch.empty calls -- workspaces, saved planes, outputs -- start non-finite."""
-    def fill():
-        held = [torch.full((n,), float("nan"), device="cuda") for n in [64, 1024, 16384, 65536, 262144] * 4]
-        held += [torch.full((n,), float("nan"), device="cuda") for n in (1 << 20, 1 << 22, 1 << 24, 1 << 26, 1 << 28)]
-        del held
-    fill()
-    yield fill
-    G.ops.set_gemm_mode("ffma")
-
-
 @pytest.fixture
 def devlib():
     """The package routed through libgnf_sm100_dev.so, whose process-global switches force a kernel; reset on the way out."""
@@ -92,57 +74,6 @@ def call(name, *args):
     lib = G._lib.lib()
     rc = getattr(lib, name)(*args, G._lib.stream_ptr())
     assert rc == 0, f"{name}: {rc} {lib.gnf_last_error()}"
-
-
-def launched(fn):
-    """Names of the CUDA kernels fn launches."""
-    from torch.profiler import ProfilerActivity, profile
-    torch.cuda.synchronize()
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        fn()
-        torch.cuda.synchronize()
-    return [e.name for e in prof.events()]
-
-
-def assert_engines(names, expect):
-    found = {k for k in ENGINES if any(k in n for n in names)}
-    assert found == set(expect), f"expected {sorted(expect)}, launched {sorted(found)}: {names}"
-
-
-class Mat:
-    """A [rows, cols] matrix of row stride ld inside a flat buffer filled with `fill`, its first element `off` floats past a
-    256-byte aligned base, one spare row after the last: padding columns and the spare row keep `fill` unless written."""
-
-    def __init__(self, rows, cols, ld, fill, off=0):
-        self.rows, self.cols, self.ld = rows, cols, ld
-        self.buf = torch.full((off + (rows + 1) * ld,), fill, device="cuda")
-        self.full = self.buf[off:].view(rows + 1, ld)
-        self.t = self.full[:rows, :cols]
-
-    @property
-    def p(self):
-        return C.c_void_p(self.full.data_ptr())
-
-    def set(self, v):
-        self.t.copy_(v)
-        return self
-
-
-def check_sentinels(out, zero_ok):
-    """Columns [cols, round_up(cols, 4)) unchanged or exactly 0 (zero_ok: forward / dgrad store 16-byte pieces), every column
-    past them and the spare row unchanged."""
-    c4 = pad4(out.cols) if zero_ok else out.cols
-    tail = out.full[:out.rows, out.cols:c4]
-    assert bool(((tail == SENT) | (tail == 0)).all()), f"columns [{out.cols}, {c4}): {tail[(tail != SENT) & (tail != 0)][:8].tolist()}"
-    rest = out.full[:out.rows, c4:]
-    assert bool((rest == SENT).all()), f"columns >= {c4} written: {rest[rest != SENT][:8].tolist()}"
-    assert bool((out.full[out.rows:] == SENT).all()), "row past the last one written"
-
-
-def cw_err(got, ref, den):
-    """max |got - ref| / den (0 where both are 0; a non-zero difference over a zero denominator is infinite)."""
-    d = (got.double() - ref).abs()
-    return float(torch.where(d == 0, torch.zeros_like(d), d / den).max()) if d.numel() else 0.
 
 
 def rel_l2(got, ref):
@@ -312,7 +243,7 @@ def check_case(case, expect, poison, seed=0, tag=""):
     case.fill("int", seed)
     poison()
     outs = []
-    assert_engines(launched(lambda: outs.extend(case.run())), expect)
+    assert_engines(launched(lambda: outs.extend(case.run())), expect, ENGINES)
     for out, (ref, _) in zip(outs, case.reference()):
         assert torch.equal(out.t.double(), ref), f"{tag}: integer operands, max err {float((out.t.double() - ref).abs().max())}"
         check_sentinels(out, zero_ok and out is outs[0])
@@ -552,7 +483,7 @@ def test_split_tf32_bits(poison, N, K, ldw, ld):
     W = Mat(N, K, ldw, NAN).set(torch.from_numpy(w).cuda())
     poison()
     out = []
-    assert_engines(launched(lambda: out.extend(split_weight(W, ld))), {SPLIT})
+    assert_engines(launched(lambda: out.extend(split_weight(W, ld))), {SPLIT}, ENGINES)
     hi, lo = out
     hi_ref = rn_tf32(w)
     lo_ref = rn_tf32(w.astype(np.float64) - hi_ref.astype(np.float64))
